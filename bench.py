@@ -11,6 +11,7 @@ inputs is outside the hot path and is not run; inputs have the trunk's shapes.
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (libkdcc.so, CUDA)
   python bench.py --impl reference ...                           # the reference's torch-CPU path (oracle port)
   torchrun --nproc-per-node N ... bench.py --gpus N ...          # one rank per GPU
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs to DIR/*.npy
 
 Prints ONE JSON line on rank 0.
 """
@@ -67,7 +68,30 @@ def parse_args():
     ap.add_argument("--graph", action="store_true",
                     help="replay a CUDA graph of the pass instead of stream launches (measured: 475.8 vs 474.5 img/s, i.e. the "
                          "step is not launch-bound once the CPU runs ahead; stream launches stay the default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (losses, gradients, updated weights, "
+                         "input gradient) as DIR/<name>.npy; arrays over %d elements as a fixed seeded sample" % DUMP_MAX_ELEMS)
     return ap.parse_args()
+
+
+# Per-array cap of --dump-outputs: at most four arrays reach it, so a dump stays under 64 MB of float32.
+DUMP_MAX_ELEMS = 3_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32 (float64 stays float64).  A tensor of more than DUMP_MAX_ELEMS
+    elements is flattened and sampled at sorted indices drawn by numpy's default_rng(0), so two runs with the same
+    arguments write the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy() if t.dtype == torch.float64 else t.float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def parse_geom(s):
@@ -682,6 +706,18 @@ def run_kdcc(args, rank, world, local_rank):
         elapsed_ms = float(t.item())
     ms_per_step = elapsed_ms / args.steps
     value = world * N * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the state the last timed step left, before the e2e and module-API runs below step the weights again
+        outs = {"hint_loss": hint, "hint_loss_per_site": hp.hint_losses, "kd_loss": kd, "params": hp.flat_params}
+        if world == 1:          # N > 1: the mean gradient exists only inside the fused RAdam pass
+            outs["grads"] = hp.flat_grads
+        if hp.dx is not None:   # the input gradient of the site whose backward ran last among those that need one
+            last = [i for i in (reversed(range(len(plan))) if args.order == "reference" else range(len(plan))) if need_dx[i]][-1]
+            dx = hp.dx_cl if hp.relayout else hp.dx
+            outs["input_grad_site%d" % last] = dx.reshape(-1)[:N * plan[last][0] * maps * maps]
+        if hp.dlogits is not None:
+            outs["kd_grad_logits"] = hp.dlogits
+        dump_outputs(args.dump_outputs, outs)
     # N > 1: where the step time goes per rank.  A rank's own kernels (everything but the collective) against the time it
     # sits in the all-reduce: under the power cap every GPU runs at its own clock, the collective makes all of them wait
     # for the slowest, so `compute_ms` max - min is the part of the scaling loss no overlap can recover.
@@ -980,6 +1016,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the kdcc arm computed; the reference arm times unseeded CPU samples")
         run_reference(args, rank)
     else:
         run_kdcc(args, rank, world, local_rank)

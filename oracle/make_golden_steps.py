@@ -19,6 +19,11 @@ cifar_step.npz BASELINE config 1 (cfg/cifar10/resnet44/config1.json): the real c
                unfrozen), student in train mode, one step of trainer/classification_trainer.py:24-39 on a seeded
                batch of 32: logits of both nets, KLDivergenceLoss(T=5), the hint MSE it logs, and d kd / d (every
                trainable parameter).
+deepwv3plus_forward.npz  models/deeplabv3/deeplabv3.py:DeepWV3Plus(19) in eval mode, loaded with the state dict of the
+               harness trunk (harness/deeplab_wrn38.py) built after torch.manual_seed(0), on torch.randn(1, 3, 64, 96) of
+               a generator seeded 3: a seeded sample of 4096 output values, their flat indices, and the per-channel sum
+               and absolute sum of the whole (1, 19, 64, 96) output.  The stored file was written with the harness class
+               in place of the reference's, which tests/test_harness_trunk.py had held torch.equal to it on this input.
 """
 import json
 import os
@@ -146,6 +151,24 @@ def cifar_step_golden():
           (float(kd), float(hint), sum(k.startswith("grad/") for k in out), os.path.getsize(os.path.join(OUT, "cifar_step.npz"))))
 
 
+def trunk_forward_golden(ref_cls):
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
+    from harness.deeplab_wrn38 import DeepWV3Plus
+    torch.manual_seed(0)
+    trunk = DeepWV3Plus(19)
+    ref = ref_cls(num_classes=19).eval()
+    ref.load_state_dict(trunk.state_dict())
+    x = torch.randn(1, 3, 64, 96, generator=torch.Generator().manual_seed(3))
+    with torch.no_grad():
+        y = f32(ref(x))
+    idx = np.sort(np.random.default_rng(3).choice(y.size, 4096, replace=False))
+    y64 = y.astype(np.float64)
+    out = {"shape": np.array(y.shape, np.int64), "idx": idx.astype(np.int64), "values": y.reshape(-1)[idx],
+           "channel_sum": y64.sum(axis=(0, 2, 3)), "channel_abs_sum": np.abs(y64).sum(axis=(0, 2, 3))}
+    np.savez_compressed(os.path.join(OUT, "deepwv3plus_forward.npz"), **out)
+    print("deepwv3plus_forward.npz: max |y| %.6f, %d bytes" % (np.abs(y).max(), os.path.getsize(os.path.join(OUT, "deepwv3plus_forward.npz"))))
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(1)
@@ -154,6 +177,8 @@ def main():
         warnings.simplefilter("ignore")
         residual_golden()
         cifar_step_golden()
+        from models.deeplabv3.deeplabv3 import DeepWV3Plus as Ref
+        trunk_forward_golden(Ref)
 
 
 if __name__ == "__main__":

@@ -1,13 +1,12 @@
 """The DeepLabV3+/WideResNet38 harness trunk (harness/deeplab_wrn38.py) keeps the reference's checkpoint layout and block
 names: key/shape listing frozen from models/deeplabv3/deeplabv3.py:DeepWV3Plus (tests/golden/deepwv3plus_keys.json, written
 by oracle/make_golden_steps.py), the survey's parameter-count known answers, and the 51M plan's surgery through the
-drop-in student wrapper.  In the build container (where /root/reference exists) the forward pass is also compared with
-the reference class itself."""
+drop-in student wrapper, and the forward pass against stored outputs of the reference class
+(tests/golden/deepwv3plus_forward.npz)."""
 import json
 import os
-import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 
@@ -42,28 +41,17 @@ def test_51m_plan_surgery_gives_the_survey_parameter_counts(trunk):
     assert not model.student.training                                            # F9: the student stays in eval mode
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference sources only exist in the build container")
 def test_forward_matches_the_reference_class(trunk):
-    cwd, path = os.getcwd(), list(sys.path)
-    try:
-        for name, attrs in (("beautifultable", {"BeautifulTable": type("BeautifulTable", (), {})}),
-                            ("torchsummary", {"summary": lambda *a, **k: None}), ("tensorboardX", {"SummaryWriter": object})):
-            if name not in sys.modules:
-                m = types.ModuleType(name)
-                m.__dict__.update(attrs)
-                sys.modules[name] = m
-        os.chdir("/root/reference")
-        sys.path.insert(0, "/root/reference")
-        saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "models" or k.startswith("models.")}
-        from models.deeplabv3.deeplabv3 import DeepWV3Plus as Ref
-        ref = Ref(num_classes=19).eval()
-        ref.load_state_dict(trunk.state_dict())
-        x = torch.randn(1, 3, 64, 96, generator=torch.Generator().manual_seed(3))
-        with torch.no_grad():
-            assert torch.equal(ref(x), trunk(x))
-    finally:
-        os.chdir(cwd)
-        sys.path[:] = path
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    # deepwv3plus_forward.npz: the reference class's output on this input and these weights (oracle/make_golden_steps.py).
+    # CPU convolutions pick their summation order by thread count and ISA: values 1e-6 of max |y| apart, channel sums
+    # 2e-8 of the largest absolute sum.  The bounds keep a 10x margin over that; a BatchNorm eps of 1e-3 instead of 1e-5
+    # in one middle unit moves the channel sums by 6e-7.
+    g = np.load(os.path.join(GOLDEN, "deepwv3plus_forward.npz"))
+    x = torch.randn(1, 3, 64, 96, generator=torch.Generator().manual_seed(3))
+    with torch.no_grad():
+        y = trunk(x).numpy()
+    assert list(y.shape) == g["shape"].tolist()
+    np.testing.assert_allclose(y.reshape(-1)[g["idx"]], g["values"], rtol=0, atol=1e-5 * float(np.abs(g["values"]).max()))
+    y64 = y.astype(np.float64)
+    np.testing.assert_allclose(y64.sum(axis=(0, 2, 3)), g["channel_sum"], rtol=0, atol=2e-7 * float(g["channel_abs_sum"].max()))
+    np.testing.assert_allclose(np.abs(y64).sum(axis=(0, 2, 3)), g["channel_abs_sum"], rtol=2e-7)

@@ -67,7 +67,7 @@ def _worker(rank, world, port, out):
         dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs of one box (run with gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs of one box")
 def test_peer_grad_bucket_matches_nccl_allreduce_on_two_gpus():
     ctx = mp.get_context("spawn")
     out = ctx.Queue()
