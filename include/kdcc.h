@@ -141,6 +141,32 @@ int kdcc_hint_loss(const void *s, const void *t, const float *w, int w_per_sampl
                    float *loss_out, void *workspace, size_t workspace_bytes, int N, int C, long HW,
                    int layout, float scale, int dtype, float grad_scale, kdcc_stream_t stream);
 
+/* kdcc_ce_loss replaces losses/CrossEntropy.py:10-15 (CrossEntropyLoss2d = NLLLoss2d(log_softmax(inputs, 1), weight, ignore_index)):
+ *   valid pixel: label in [0, C) and != ignore_index;  w = weight[label] (weight NULL -> 1)
+ *   *loss_out = sum_valid w * (logsumexp_c s - s_label) / (mean ? sum_valid w : 1)   (mean with no valid pixel -> NaN, as torch)
+ *   ds        = grad_scale * w * (softmax(s) - onehot(label)) / (mean ? sum_valid w : 1); 0 at invalid pixels; NULL: skip
+ * Logit strides as kdcc_kd_loss (NCHW and channels_last without copies); labels int64 [N][HW]; weight fp32 [C]; C <= 32.
+ * In mean mode with ds, a pre-pass over the labels forms the normaliser so that ds is written once, already normalised.
+ * bad_labels (nullable, device int64) += number of labels outside [0, C) that are not ignore_index: they are dropped,
+ * never used as an index (torch would stop with a device-side assert). */
+size_t kdcc_ce_workspace_bytes(int N, long HW);
+int kdcc_ce_loss(const void *s, const long long *labels, const float *weight, int ignore_index, int mean,
+                 void *ds, float *loss_out, long long *bad_labels, void *workspace, size_t workspace_bytes,
+                 int N, int C, long HW, long batch_stride, long class_stride, long pixel_stride,
+                 int dtype, float grad_scale, kdcc_stream_t stream);
+
+/* kdcc_logits_stats: the logged-only quantities of one layerwise step (trainer/layerwise_trainer.py:225-227,244-250) in ONE
+ * read of s, t and the labels, no gradients:
+ *   out3[0] = KD term: kd_mode 0 none (untouched), 1 = kdcc_kd_loss value (temperature T), 2 = MSELoss value x kd_scale
+ *   out3[1] = CE(s, labels), out3[2] = CE(t, labels)   (as kdcc_ce_loss, same weight / ignore / mean)
+ *   conf_s / conf_t (nullable, int64 [C*C], accumulated) += confusion of argmax(s) / argmax(t), exactly as kdcc_confusion_update.
+ * s and t share dtype and strides.  t may be NULL (validation: student only; out3[0], out3[2], conf_t untouched, kd_mode
+ * ignored).  With kd_mode 1 and T == 1 the KD term reuses the CE exponentials.  Workspace: kdcc_ce_workspace_bytes. */
+int kdcc_logits_stats(const void *s, const void *t, const long long *labels, const float *weight, int ignore_index, int mean,
+                      int kd_mode, float T, float kd_scale, float *out3, long long *conf_s, long long *conf_t,
+                      long long *bad_labels, void *workspace, size_t workspace_bytes, int N, int C, long HW,
+                      long batch_stride, long class_stride, long pixel_stride, int dtype, kdcc_stream_t stream);
+
 /* ---- small utilities used by the host mirror so no torch arithmetic sits on the path ------------ */
 /* dst_bf16[i] = bf16(src_f32[i]) */
 int kdcc_cast_f32_to_bf16(const float *src, void *dst, long n, kdcc_stream_t stream);

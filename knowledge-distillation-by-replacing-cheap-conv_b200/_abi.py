@@ -33,6 +33,10 @@ SIGNATURES = {
     "kdcc_kd_loss": (_i, [_vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l, _f, _i, _i, _f, _vp]),
     "kdcc_kd_loss_multi": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l, _f, _i, _f, _vp]),
     "kdcc_hint_loss": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _sz, _i, _i, _l, _i, _f, _i, _f, _vp]),
+    "kdcc_ce_workspace_bytes": (_sz, [_i, _l]),
+    "kdcc_ce_loss": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l, _i, _f, _vp]),
+    "kdcc_logits_stats": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l,
+                               _i, _vp]),
     "kdcc_cast_f32_to_bf16": (_i, [_vp, _vp, _l, _vp]),
     "kdcc_scale_inplace": (_i, [_vp, _vp, _l, _i, _vp]),
     "kdcc_scale_inplace_expect": (_i, [_vp, _vp, _f, _l, _i, _vp]),

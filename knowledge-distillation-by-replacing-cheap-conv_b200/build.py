@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libkdcc.so")
 
-SOURCES = ["loss_kernels.cu", "layout_convert.cu", "metrics.cu", "tta.cu", "optim.cu", "dw_direct.cu", "dw_tma.cu", "dw_nhwc3.cu", "dw_tc.cu", "dw_tc2.cu", "dw_tc_wgrad.cu", "dw_tc_wgrad2.cu", "dw_tc_wgrad3.cu", "dw_api.cu", "pw_gemm_sm100.cu", "pw_gemm_simt.cu",
+SOURCES = ["loss_kernels.cu", "ce_kernels.cu", "layout_convert.cu", "metrics.cu", "tta.cu", "optim.cu", "dw_direct.cu", "dw_tma.cu", "dw_nhwc3.cu", "dw_tc.cu", "dw_tc2.cu", "dw_tc_wgrad.cu", "dw_tc_wgrad2.cu", "dw_tc_wgrad3.cu", "dw_api.cu", "pw_gemm_sm100.cu", "pw_gemm_simt.cu",
            "pw_api.cu", "tma_host.cu", "api_misc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr"]

@@ -9,6 +9,8 @@ Reference call sites replaced (reference file:line):
   pointwise_conv      models/students/transform_blocks/depthwise_separable_conv.py:13
   kd_loss             losses/KLDiv.py:19-23, losses/EnsembleKLDiv.py:18-22
   hint_loss           losses/WeightedHintMSELoss.py:12-16, losses/MSELoss.py:14-16
+  cross_entropy       losses/CrossEntropy.py:10-15
+  logits_stats        trainer/layerwise_trainer.py:225-227,244-250 (logged losses + confusion matrices, one pass)
 """
 import os
 
@@ -523,6 +525,108 @@ def hint_loss(inputs, targets, filter_weight=None, scale=1.0, expected_upstream=
     """scale/N * sum_n [sum_c w mean_hw (s-t)^2 / sum_c w]; filter_weight None = uniform (MSELoss).
     `expected_upstream`: see kd_loss."""
     return _HintLoss.apply(inputs, targets, filter_weight, float(scale), float(expected_upstream))
+
+
+def _ce_operands(s, target, weight, bad_labels):
+    """(s dense NCHW or channels_last, int64 labels (N*HW), fp32 weight or None, geometry) for the CE entry points."""
+    if s.dim() < 2:
+        raise _abi.KdccError("cross entropy expects (N, C, ...) logits, got %s" % (tuple(s.shape),))
+    s = s.detach()
+    if not (s.dim() == 4 and s.is_contiguous(memory_format=torch.channels_last) and not s.is_contiguous()):
+        s = s.contiguous()
+    geo = _logit_strides(s)
+    N, C, HW = geo[0], geo[1], geo[2]
+    target = target.detach()
+    if target.dtype != torch.int64:
+        target = target.long()
+    target = target.contiguous()
+    if target.numel() != N * HW:
+        raise _abi.KdccError("labels have %d elements, logits describe %d pixels" % (target.numel(), N * HW))
+    w = None
+    if weight is not None:
+        w = weight.detach().float().contiguous()
+        if w.numel() != C:
+            raise _abi.KdccError("class weight has %d entries, logits have %d classes" % (w.numel(), C))
+    if bad_labels is not None and (bad_labels.dtype != torch.int64 or bad_labels.numel() != 1):
+        raise _abi.KdccError("bad_labels must be a one-element int64 device tensor")
+    return s, target, w, geo
+
+
+class _CeLoss(torch.autograd.Function):
+    @staticmethod
+    @_device_guard
+    def forward(ctx, s, target, weight, ignore_index, mean, expected, bad_labels):
+        _require_cuda(s, target, weight, bad_labels)
+        s, target, w, (N, C, HW, bs, cs, ps) = _ce_operands(s, target, weight, bad_labels)
+        ds = torch.empty_like(s) if ctx.needs_input_grad[0] else None
+        loss = torch.empty((), dtype=torch.float32, device=s.device)
+        L = _abi.lib()
+        ws = _workspace(L.kdcc_ce_workspace_bytes(N, HW), s.device)
+        _abi.check(L.kdcc_ce_loss(_ptr(s), _ptr(target), _ptr(w), int(ignore_index), int(bool(mean)), _ptr(ds), _ptr(loss),
+                                  _ptr(bad_labels), _ptr(ws), ws.numel(), N, C, HW, bs, cs, ps, _dtype_code(s), float(expected),
+                                  _stream()), "kdcc_ce_loss")
+        ctx.ds = ds
+        ctx.expected = float(expected)
+        return loss
+
+    @staticmethod
+    @_device_guard
+    def backward(ctx, g):
+        ds = _take_grad(ctx)
+        if ds is None:
+            return None, None, None, None, None, None, None
+        g = g.detach().float().contiguous()
+        _abi.check(_abi.lib().kdcc_scale_inplace_expect(_ptr(ds), _ptr(g), ctx.expected, ds.numel(), _dtype_code(ds), _stream()),
+                   "kdcc_scale_inplace_expect")
+        return ds, None, None, None, None, None, None
+
+
+def cross_entropy(logits, target, weight=None, ignore_index=255, mean=True, expected_upstream=1.0, bad_labels=None):
+    """losses/CrossEntropy.py:10-15: NLL of log_softmax(logits, 1) at the labels, weighted by weight[label], over the
+    pixels whose label is a class index other than ignore_index; mean=True divides by the summed weight (NaN when no
+    pixel counts, as torch), mean=False returns the sum.  fp32 0-dim tensor with grad_fn; one kernel pass (plus a
+    pre-pass over the labels when a mean-mode gradient is needed).  Labels outside [0, C) other than ignore_index are
+    dropped, never used as an index, and added to `bad_labels` (one-element int64 device tensor) when given.
+    `expected_upstream`: see kd_loss."""
+    return _CeLoss.apply(logits, target, weight, int(ignore_index), bool(mean), float(expected_upstream), bad_labels)
+
+
+def _conf_arg(conf, C):
+    if conf is None:
+        return None
+    _require_cuda(conf)
+    if conf.dtype != torch.int64 or not conf.is_contiguous() or conf.numel() != C * C:
+        raise _abi.KdccError("confusion accumulator must be a contiguous int64 tensor of %d cells" % (C * C))
+    return conf
+
+
+@torch.no_grad()
+@_device_guard
+def logits_stats(s, t, target, weight=None, ignore_index=255, mean=True, kd_mode=0, temperature=1.0, kd_scale=1.0,
+                 conf_s=None, conf_t=None, bad_labels=None):
+    """The logged-only quantities of one layerwise step (trainer/layerwise_trainer.py:225-227,244-250) in one pass over
+    the student logits `s`, the teacher logits `t` and the labels: returns (kd, ce_s, ce_t), 0-dim fp32 device tensors
+    (views of one buffer; nothing is read back to the host).
+      kd   = kd_mode 1: KLDivergenceLoss(temperature)(s, t); 2: MSELoss(num_classes=kd_scale)(s, t); 0: None
+      ce_s = cross_entropy(s, target, weight, ignore_index, mean), ce_t the same for t
+    conf_s / conf_t (int64 C*C, device) += the confusion matrices of argmax(s) / argmax(t), as confusion_update.
+    t=None (validation): only ce_s and conf_s; kd and ce_t are None."""
+    _require_cuda(s, t, target, weight, conf_s, conf_t, bad_labels)
+    s, target, w, (N, C, HW, bs, cs, ps) = _ce_operands(s, target, weight, bad_labels)
+    if t is not None:
+        if t.shape != s.shape:
+            raise _abi.KdccError("logits_stats expects matching (N, C, ...) tensors, got %s and %s" % (tuple(s.shape), tuple(t.shape)))
+        t = t.detach().to(s.dtype).contiguous(memory_format=torch.channels_last if ps != 1 else torch.contiguous_format)
+    else:
+        kd_mode, conf_t = 0, None
+    conf_s, conf_t = _conf_arg(conf_s, C), _conf_arg(conf_t, C)
+    out3 = torch.empty(3, dtype=torch.float32, device=s.device)
+    L = _abi.lib()
+    ws = _workspace(L.kdcc_ce_workspace_bytes(N, HW), s.device)
+    _abi.check(L.kdcc_logits_stats(_ptr(s), _ptr(t), _ptr(target), _ptr(w), int(ignore_index), int(bool(mean)), int(kd_mode),
+                                   float(temperature), float(kd_scale), _ptr(out3), _ptr(conf_s), _ptr(conf_t), _ptr(bad_labels),
+                                   _ptr(ws), ws.numel(), N, C, HW, bs, cs, ps, _dtype_code(s), _stream()), "kdcc_logits_stats")
+    return (out3[0] if kd_mode else None), out3[1], (out3[2] if t is not None else None)
 
 
 # ---------------------------------------------------------------------------------------------------

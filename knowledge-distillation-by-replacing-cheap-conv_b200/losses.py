@@ -13,6 +13,24 @@ from . import functional as F_kdcc
 # differ), which removes a full read-modify-write pass over the gradient from every backward.  Not a reference argument.
 
 
+class CrossEntropyLoss2d(nn.Module):
+    """losses/CrossEntropy.py:7-15 -- NLLLoss2d(log_softmax(inputs, 1), weight, size_average, ignore_index): weighted mean
+    (size_average True or None) or sum of the per-pixel NLL over the pixels whose label is not ignore_index.  The value
+    and the gradient come from one kernel pass; labels outside [0, C) other than ignore_index are dropped instead of
+    stopping the device."""
+
+    def __init__(self, weight=None, size_average=True, ignore_index=255):
+        super().__init__()
+        self.register_buffer("weight", weight)   # as NLLLoss2d: follows the module to the device
+        self.size_average = size_average
+        self.ignore_index = ignore_index
+        self.expected_upstream = 1.0
+
+    def forward(self, inputs, targets):
+        return F_kdcc.cross_entropy(inputs, targets, self.weight, self.ignore_index, mean=self.size_average is not False,
+                                    expected_upstream=self.expected_upstream)
+
+
 class KLDivergenceLoss(nn.Module):
     """losses/KLDiv.py:4-23 -- kl_div(log_softmax(s/T), softmax(t/T)) * T^2 * C, 'mean' over all elements."""
 

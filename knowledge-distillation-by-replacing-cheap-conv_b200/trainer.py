@@ -16,6 +16,8 @@ from functools import reduce
 import torch
 
 from .metrics import ConfusionMatrix  # noqa: F401  (kernel-backed; kept importable from here)
+from . import functional as F_kdcc
+from .losses import CrossEntropyLoss2d, KLDivergenceLoss, MSELoss
 import torch.distributed as dist
 
 
@@ -111,16 +113,28 @@ def _expect(criterion, value):
         criterion.expected_upstream = float(value)
 
 
+def _confusion_of(metric):
+    """(int64 C*C device matrix, ignore_index) behind a ConfusionMatrix / CityscapesMetricTracker."""
+    cm = getattr(metric, "_cm", metric)
+    return cm.mat, cm.ignore
+
+
 class LayerwiseStep:
-    """criterions = [supervised, kd, hint] as in train.py:48-50; `model` is a DepthwiseStudent."""
+    """criterions = [supervised, kd, hint] as in train.py:48-50; `model` is a DepthwiseStudent.
+
+    `metrics` (optional): a (student, teacher) pair of kdcc ConfusionMatrix / CityscapesMetricTracker updated with the
+    step's logits (trainer/layerwise_trainer.py:247-250).  When criterions[0] is a kdcc CrossEntropyLoss2d, the logged
+    supervised / teacher CE, the KD term (kdcc KLDivergenceLoss or MSELoss; any other criterion is called as it is) and
+    both confusion matrices come from ONE pass over the two logit tensors and the labels (kdcc_logits_stats)."""
 
     def __init__(self, model, criterions, optimizer, accumulation_steps=1, process_group=None, log_supervised=True,
-                 peer_exchange=True):
+                 peer_exchange=True, metrics=None):
         self.model, self.criterions, self.optimizer = model, criterions, optimizer
         self.accumulation_steps = int(accumulation_steps)
         self.group = process_group
         self.log_supervised = log_supervised
         self.peer_exchange = peer_exchange
+        self.metrics = metrics
         self.bucket = None
         self.rebuild_bucket()
         _expect(criterions[2], 1.0 / self.accumulation_steps)   # loss = sum(hint pairs) / accumulation_steps
@@ -138,12 +152,18 @@ class LayerwiseStep:
         pairs = list(zip(self.model.student_hidden_outputs, self.model.teacher_hidden_outputs))
         hint_loss = reduce(lambda a, st: a + self.criterions[2](st[0], st[1]), pairs, 0) / acc
         with torch.no_grad():  # logged, never back-propagated by this trainer
-            kd_loss = self.criterions[1](output_st, output_tc) / acc
-            if self.log_supervised and target is not None:
-                supervised = self.criterions[0](output_st, target) / acc
-                teacher_loss = self.criterions[0](output_tc, target)
+            if self.log_supervised and target is not None and isinstance(self.criterions[0], CrossEntropyLoss2d):
+                kd_loss, supervised, teacher_loss = self._fused_stats(output_st, output_tc, target)
             else:
-                supervised = teacher_loss = torch.zeros((), device=data.device)
+                kd_loss = self.criterions[1](output_st, output_tc) / acc
+                if self.log_supervised and target is not None:
+                    supervised = self.criterions[0](output_st, target) / acc
+                    teacher_loss = self.criterions[0](output_tc, target)
+                else:
+                    supervised = teacher_loss = torch.zeros((), device=data.device)
+                if self.metrics is not None and target is not None:
+                    self.metrics[0].update(output_st, target)
+                    self.metrics[1].update(output_tc, target)
         loss = hint_loss
         if torch.is_tensor(loss):
             loss.backward()
@@ -153,6 +173,31 @@ class LayerwiseStep:
             self.bucket.zero()  # == optimizer.zero_grad() for the trainable set, keeps the flat views alive
         return {"loss": loss, "hint_loss": hint_loss, "kd_loss": kd_loss, "supervised_loss": supervised,
                 "teacher_loss": teacher_loss, "output_st": output_st.detach(), "output_tc": output_tc}
+
+    def _fused_stats(self, output_st, output_tc, target):
+        """(kd / acc, supervised / acc, teacher) of one kdcc_logits_stats pass; confusion matrices that do not share the
+        criterion's ignore_index or class count are updated by their own pass."""
+        acc = self.accumulation_steps
+        ce, kd_crit = self.criterions[0], self.criterions[1]
+        kd_mode, T, scale = 0, 1.0, 1.0
+        if isinstance(kd_crit, KLDivergenceLoss):
+            kd_mode, T = 1, float(kd_crit.temperature)
+        elif isinstance(kd_crit, MSELoss):
+            kd_mode, scale = 2, float(kd_crit.num_classes)
+        confs, separate = [None, None], []
+        for i, (metric, logits) in enumerate(zip(self.metrics or (), (output_st, output_tc))):
+            mat, ignore = _confusion_of(metric)
+            if ignore == ce.ignore_index and mat.numel() == logits.shape[1] ** 2:
+                confs[i] = mat
+            else:
+                separate.append((metric, logits))
+        kd, sup, tea = F_kdcc.logits_stats(output_st, output_tc, target, ce.weight, ce.ignore_index,
+                                           mean=ce.size_average is not False, kd_mode=kd_mode, temperature=T, kd_scale=scale,
+                                           conf_s=confs[0], conf_t=confs[1])
+        for metric, logits in separate:
+            metric.update(logits, target)
+        kd_loss = (kd if kd_mode else kd_crit(output_st, output_tc)) / acc
+        return kd_loss, sup / acc, tea
 
 
 class ClassificationStep:
@@ -205,6 +250,7 @@ class EnsembleStep:
         self.accumulation_steps, self.weight, self.kd_multi = int(accumulation_steps), weight, kd_multi
         self.group = process_group
         self.bucket = GradBucket(model.trainable_parameters())
+        _expect(criterions[0], 1.0 / self.accumulation_steps)   # loss = kd + supervised / accumulation_steps
 
     def rebuild_bucket(self):
         self.bucket = GradBucket(self.model.trainable_parameters())
