@@ -167,6 +167,24 @@ int kdcc_logits_stats(const void *s, const void *t, const long long *labels, con
                       long long *bad_labels, void *workspace, size_t workspace_bytes, int N, int C, long HW,
                       long batch_stride, long class_stride, long pixel_stride, int dtype, kdcc_stream_t stream);
 
+/* kdcc_ensemble_loss: the objective of trainer/ensemble_trainer.py:73-90 (loss = kd + supervised) in ONE pass that reads
+ * s once, each of the K (1..8) teachers once and the labels once:
+ *   out3[0] = sum_k kd_weights[k] * T^2/(N*HW) * sum_pix KL(softmax(t_k/T) || softmax(s/T))   (as kdcc_kd_loss_multi)
+ *   out3[1] = CE(s, labels) as kdcc_ce_loss (class_weight, ignore_index, mean; NaN for a mean over no valid pixel)
+ *   out3[2] = D, the CE normaliser: sum_valid class_weight[label] in mean mode, 1 in sum mode
+ *   ds      = e_kd * T/(N*HW) * ((sum_k w_k) softmax(s/T) - sum_k w_k softmax(t_k/T))
+ *           + e_ce * class_weight[label] * (softmax(s) - onehot(label)) / D      (CE part 0 at dropped pixels)
+ * written once (NULL: values only).  (e_kd, e_ce) = (kd_grad_scale, ce_grad_scale), the upstream pair the caller expects.
+ * teachers / kd_weights are HOST arrays (copied into the kernel parameters); all logits share dtype and strides; C <= 32.
+ * upstream2 != NULL (device, fp32 [2] = the actual (g_kd, g_ce)): gradient-only re-launch after a forward call with the same
+ * arguments -- every CTA returns at once when the pair equals (kd_grad_scale, ce_grad_scale); otherwise ds is rewritten
+ * with the actual pair and the D of out3[2].  Workspace: kdcc_ce_workspace_bytes. */
+int kdcc_ensemble_loss(const void *s, const void *const *teachers, const float *kd_weights, int K, float T,
+                       const long long *labels, const float *class_weight, int ignore_index, int mean,
+                       void *ds, float *out3, long long *bad_labels, void *workspace, size_t workspace_bytes,
+                       int N, int C, long HW, long batch_stride, long class_stride, long pixel_stride, int dtype,
+                       float kd_grad_scale, float ce_grad_scale, const float *upstream2, kdcc_stream_t stream);
+
 /* ---- small utilities used by the host mirror so no torch arithmetic sits on the path ------------ */
 /* dst_bf16[i] = bf16(src_f32[i]) */
 int kdcc_cast_f32_to_bf16(const float *src, void *dst, long n, kdcc_stream_t stream);

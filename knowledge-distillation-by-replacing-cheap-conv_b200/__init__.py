@@ -7,12 +7,12 @@ Host-side mirror of the reference's module interfaces over the C-ABI library lib
 from . import _abi
 from ._abi import KdccError, LIB_PATH
 from .blocks import DepthwiseSeparableBlock
-from .losses import CrossEntropyLoss2d, EnsembleKLDivergenceLoss, KLDivergenceLoss, MSELoss, MultiTeacherKLDivergenceLoss, WeightedHintMSELoss
+from .losses import CrossEntropyLoss2d, EnsembleDistillationLoss, EnsembleKLDivergenceLoss, KLDivergenceLoss, MSELoss, MultiTeacherKLDivergenceLoss, WeightedHintMSELoss
 from . import checkpoint, functional, optim, tta
 from .student import DepthwiseStudent
 from .metrics import CityscapesMetricTracker, ConfusionMatrix
 from .trainer import ClassificationStep, EnsembleStep, GradBucket, LayerwiseStep, prepare_train_epoch
 from .peer_reduce import PeerGradBucket
 
-__all__ = ["DepthwiseSeparableBlock", "DepthwiseStudent", "LayerwiseStep", "ClassificationStep", "EnsembleStep", "GradBucket", "PeerGradBucket", "prepare_train_epoch", "ConfusionMatrix", "CityscapesMetricTracker", "CrossEntropyLoss2d", "KLDivergenceLoss", "EnsembleKLDivergenceLoss", "MultiTeacherKLDivergenceLoss", "MSELoss", "WeightedHintMSELoss",
+__all__ = ["DepthwiseSeparableBlock", "DepthwiseStudent", "LayerwiseStep", "ClassificationStep", "EnsembleStep", "GradBucket", "PeerGradBucket", "prepare_train_epoch", "ConfusionMatrix", "CityscapesMetricTracker", "CrossEntropyLoss2d", "EnsembleDistillationLoss", "KLDivergenceLoss", "EnsembleKLDivergenceLoss", "MultiTeacherKLDivergenceLoss", "MSELoss", "WeightedHintMSELoss",
            "functional", "checkpoint", "KdccError", "LIB_PATH"]

@@ -37,6 +37,8 @@ SIGNATURES = {
     "kdcc_ce_loss": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l, _i, _f, _vp]),
     "kdcc_logits_stats": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l,
                                _i, _vp]),
+    "kdcc_ensemble_loss": (_i, [_vp, _vp, _vp, _i, _f, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz, _i, _i, _l, _l, _l, _l,
+                                _i, _f, _f, _vp, _vp]),
     "kdcc_cast_f32_to_bf16": (_i, [_vp, _vp, _l, _vp]),
     "kdcc_scale_inplace": (_i, [_vp, _vp, _l, _i, _vp]),
     "kdcc_scale_inplace_expect": (_i, [_vp, _vp, _f, _l, _i, _vp]),

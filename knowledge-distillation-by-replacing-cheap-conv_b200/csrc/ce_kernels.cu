@@ -3,7 +3,9 @@
 //                        ignore_index)): value and gradient in one pass over the logits
 //   logits_stats_kernel  trainer/layerwise_trainer.py:225-227,244-250: CE(student), CE(teacher), the KD term and both
 //                        confusion matrices in ONE read of the two logit tensors and the labels, no gradient
-// Both are HBM-bound and follow loss_kernels.cu: logits in registers ([CT][PIX], two pixels per thread on class planes),
+//   ensemble_loss_kernel trainer/ensemble_trainer.py:73-90: multi-teacher KD + CE and one gradient of their sum in ONE
+//                        pass over the student logits, every teacher and the labels
+// All are HBM-bound and follow loss_kernels.cu: logits in registers ([CT][PIX], two pixels per thread on class planes),
 // fp32 math with exp2 / log2, a fixed-order block reduction into per-CTA partials and a one-block double finalize, so
 // every scalar is bit-reproducible run to run.  Confusion counts are integers (shared-memory atomics, as metrics.cu).
 #include "loss_common.cuh"
@@ -293,14 +295,176 @@ __global__ void __launch_bounds__(kLossThreads, CT <= 19 ? 2 : 1) logits_stats_k
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// The objective of the ensemble loop (trainer/ensemble_trainer.py:73-90, loss = kd + supervised) in ONE pass over the
+// student logits: every teacher is read once (kd_multi_kernel's register-resident softmax), the labels once, and
+//   kd  = sum_k w_k T^2/(N*HW) sum_pix KL(softmax(t_k/T) || softmax(s/T))      (partials: kSlotKd, in bits)
+//   ce  = sum_valid cw * (logsumexp s - s_label)                                 (partials: kSlotCeS / kSlotW)
+//   ds  = e_kd T/(N*HW) ((sum_k w_k) softmax(s/T) - sum_k w_k softmax(t_k/T)) + e_ce cw (softmax(s) - onehot) / D
+// written once.  With T == 1 the CE exponentials are the KD student exponentials.
+// ------------------------------------------------------------------------------------------------
+constexpr int kEnsMaxTeachers = 8;
+struct EnsParams {
+  const void *s;
+  const void *t[kEnsMaxTeachers];
+  float w[kEnsMaxTeachers];
+  float wsum;
+  int K;
+  const long long *labels;
+  const float *weight;         // class weights fp32 [C] or nullptr (all 1)
+  void *ds;
+  float *part;                 // [kCeSlots][stride]; nullptr on a gradient-only re-launch
+  long stride;
+  const float *den;            // D on the device (mean-mode label pre-pass, or out3[2]), or nullptr: D = 1
+  const float *up2;            // re-launch: the actual upstream pair (g_kd, g_ce) on the device, else nullptr
+  float e_kd, e_ce;            // the upstream pair folded into ds (forward) / expected (re-launch)
+  unsigned long long *bad;
+  long HW, bs, cs, ps;
+  long groups, HWg;
+  int C, ignore;
+  int shared;                  // T == 1
+  float k2;                    // log2(e) / T
+  float kd_g;                  // T / (N*HW)
+};
+
+template <typename T, int CT, bool EXACT, int PIX, bool GRAD>
+__global__ void __launch_bounds__(kLossThreads, CT <= 19 ? 2 : 1) ensemble_loss_kernel(const EnsParams p) {
+  float e_kd = p.e_kd, e_ce = p.e_ce;
+  if (GRAD && p.up2 != nullptr) {
+    // gradient-only re-launch: the forward already wrote ds for the expected pair; every CTA leaves when it was right
+    e_kd = __ldg(p.up2);
+    e_ce = __ldg(p.up2 + 1);
+    if (e_kd == p.e_kd && e_ce == p.e_ce) return;
+  }
+  __shared__ float scratch[32];
+  __shared__ float wsh[kCeMaxC];
+  __shared__ unsigned int bad_sh;
+  const T *__restrict__ sbase = static_cast<const T *>(p.s);
+  T *__restrict__ dbase = static_cast<T *>(p.ds);
+  const int C = EXACT ? CT : p.C;
+  ce_load_weights(p.weight, C, wsh);
+  if (threadIdx.x == 0) bad_sh = 0u;
+  __syncthreads();
+  const float cc = GRAD ? e_ce / (p.den != nullptr ? __ldg(p.den) : 1.f) : 0.f;
+  const float kc = GRAD ? e_kd * p.kd_g : 0.f;
+  float lsum = 0.f, wsum = 0.f, kd = 0.f;
+  int bad = 0;
+  for (long g = (long)blockIdx.x * blockDim.x + threadIdx.x; g < p.groups; g += (long)gridDim.x * blockDim.x) {
+    const long n = g / p.HWg;
+    const long q = (g - n * p.HWg) * PIX;
+    const long off = n * p.bs + q * p.ps;
+    // sv: log2 softmax(s/T); gd: the gradient, built up teacher by teacher; kl: sum_k w_k KL_k in bits
+    float sv[CT][PIX], gd[GRAD ? CT : 1][PIX], kl[PIX];
+#pragma unroll
+    for (int c = 0; c < CT; ++c)
+      if (EXACT || c < C) load_pix<T, PIX>(sbase + off + c * p.cs, sv[c]);
+    long long lab[PIX];
+    load_labels<PIX>(p.labels + n * p.HW + q, lab);
+#pragma unroll
+    for (int i = 0; i < PIX; ++i) {
+      float w;
+      const int cls = ce_class(lab[i], C, p.ignore, wsh, w, bad);
+      float smax = -INFINITY;
+#pragma unroll
+      for (int c = 0; c < CT; ++c)
+        if (EXACT || c < C) smax = fmaxf(smax, sv[c][i]);
+      // e1 = 2^a (CE, kept in gd), e2 = 2^(a/T) (KD): the same exponential when T == 1
+      float e2[CT];
+      float s1 = 0.f, s2 = 0.f, alab = 0.f;
+#pragma unroll
+      for (int c = 0; c < CT; ++c)
+        if (EXACT || c < C) {
+          const float d = sv[c][i] - smax;
+          const float a = d * kLog2e;
+          const float e1 = exp2f(a);
+          s1 += e1;
+          if (c == cls) alab = a;
+          e2[c] = p.shared ? e1 : exp2f(d * p.k2);
+          s2 += e2[c];
+          sv[c][i] = d * p.k2;
+          if (GRAD) gd[c][i] = e1;
+        }
+      if (cls >= 0) {
+        lsum += w * (log2f(s1) - alab);
+        wsum += w;
+      }
+      const float l2 = log2f(s2), r2 = 1.f / s2, r1 = 1.f / s1;
+      const float gw = cls >= 0 ? cc * w : 0.f;   // the CE part is exactly 0 at dropped pixels
+#pragma unroll
+      for (int c = 0; c < CT; ++c)
+        if (EXACT || c < C) {
+          if (GRAD) gd[c][i] = kc * p.wsum * (e2[c] * r2) + gw * (gd[c][i] * r1 - (c == cls ? 1.f : 0.f));
+          sv[c][i] -= l2;
+        }
+      kl[i] = 0.f;
+    }
+    for (int k = 0; k < p.K; ++k) {
+      const T *__restrict__ tbase = static_cast<const T *>(p.t[k]);
+      const float wk = p.w[k];
+      float tv[CT][PIX];
+#pragma unroll
+      for (int c = 0; c < CT; ++c)
+        if (EXACT || c < C) load_pix<T, PIX>(tbase + off + c * p.cs, tv[c]);
+#pragma unroll
+      for (int i = 0; i < PIX; ++i) {
+        float tmax = -INFINITY;
+#pragma unroll
+        for (int c = 0; c < CT; ++c)
+          if (EXACT || c < C) tmax = fmaxf(tmax, tv[c][i]);
+        // one exponential per teacher logit: KL_k bits = (sum_c e b) / Z - log2 Z - (sum_c e log2 p_s) / Z
+        float tsum = 0.f, tb = 0.f;
+#pragma unroll
+        for (int c = 0; c < CT; ++c)
+          if (EXACT || c < C) {
+            const float b = (tv[c][i] - tmax) * p.k2;
+            const float et = exp2f(b);
+            tsum += et;
+            if (et > 0.f) tb += et * b;   // p == 0 contributes 0 (xlogy)
+            tv[c][i] = et;
+          }
+        const float rt = 1.f / tsum;
+        const float wr = wk * rt, gk = -kc * wr;
+        float xs = 0.f;
+#pragma unroll
+        for (int c = 0; c < CT; ++c)
+          if (EXACT || c < C) {
+            if (tv[c][i] > 0.f) xs += tv[c][i] * sv[c][i];
+            if (GRAD) gd[c][i] = fmaf(gk, tv[c][i], gd[c][i]);
+          }
+        kl[i] += wk * (tb * rt - log2f(tsum)) - wr * xs;
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < PIX; ++i) kd += kl[i];
+    if (GRAD) {
+#pragma unroll
+      for (int c = 0; c < CT; ++c)
+        if (EXACT || c < C) store_pix<T, PIX>(dbase + off + c * p.cs, gd[c]);
+    }
+  }
+  if (p.part == nullptr) return;   // uniform: a re-launch writes the gradient only
+  ce_count_bad(bad, &bad_sh);
+  const float r0 = block_sum(lsum, scratch);
+  const float r1 = block_sum(wsum, scratch);
+  const float r2 = block_sum(kd, scratch);
+  if (threadIdx.x == 0) {
+    p.part[kSlotCeS * p.stride + blockIdx.x] = r0;
+    p.part[kSlotW * p.stride + blockIdx.x] = r1;
+    p.part[kSlotKd * p.stride + blockIdx.x] = r2;
+    if (bad_sh && p.bad != nullptr) atomicAdd(p.bad, (unsigned long long)bad_sh);
+  }
+}
+
 // Fixed-order double sums of the per-CTA partials and the scalars made from them.
 struct CeFinal {
   const float *part;
   long stride;
   int count;
-  int mode;          // 0: gradient coefficient of the pre-pass, 1: CE loss, 2: logits statistics
+  int mode;          // 0: gradient coefficient of the pre-pass, 1: CE loss, 2: logits statistics,
+                     // 3: normaliser of the pre-pass (sum_valid w), 4: ensemble objective
   unsigned slots;    // bit k: slot k was written
   int mean;
+  int den_done;      // mode 4: out[2] already holds the D of the pre-pass
   double gscale;     // mode 0: grad_scale
   double kd_coef;    // mode 2: scale of the KD partial sum
   float *out;
@@ -331,6 +495,12 @@ __global__ void __launch_bounds__(256) ce_finalize_kernel(const CeFinal f) {
     f.out[0] = (float)(f.gscale / tot[kSlotPre]);
   } else if (f.mode == 1) {
     f.out[0] = (float)(ln2 * tot[kSlotCeS] / den);
+  } else if (f.mode == 3) {
+    f.out[0] = (float)tot[kSlotPre];
+  } else if (f.mode == 4) {
+    f.out[0] = (float)(f.kd_coef * tot[kSlotKd]);
+    f.out[1] = (float)(ln2 * tot[kSlotCeS] / den);
+    if (!f.den_done) f.out[2] = (float)den;
   } else {
     f.out[1] = (float)(ln2 * tot[kSlotCeS] / den);
     if (f.slots & (1u << kSlotCeT)) f.out[2] = (float)(ln2 * tot[kSlotCeT] / den);
@@ -419,6 +589,101 @@ KDCC_API int kdcc_ce_loss(const void *s, const long long *labels, const float *w
   CeFinal f{};
   f.part = p.part; f.stride = p.stride; f.count = grid; f.mode = 1;
   f.slots = (1u << kSlotCeS) | (1u << kSlotW); f.mean = mean; f.out = loss_out;
+  launch_pdl(ce_finalize_kernel, dim3(1), dim3(256), 0, st, f);
+  return launch_status();
+}
+
+template <typename T, bool GRAD>
+static void launch_ensemble(const EnsParams &p, bool vec2, int grid, cudaStream_t st) {
+// two pixels per thread only for the 10-class planes: with three C x PIX register arrays the 16 / 19 / 32 forms would spill
+#define ENS_LAUNCH(CT, EXACT)                                                                                   \
+  do {                                                                                                          \
+    if constexpr (CT == 10) {                                                                                   \
+      if (vec2) { ensemble_loss_kernel<T, CT, EXACT, 2, GRAD><<<grid, kLossThreads, 0, st>>>(p); break; }       \
+    }                                                                                                           \
+    ensemble_loss_kernel<T, CT, EXACT, 1, GRAD><<<grid, kLossThreads, 0, st>>>(p);                              \
+  } while (0)
+  if (p.C == 19) ENS_LAUNCH(19, true);
+  else if (p.C == 10) ENS_LAUNCH(10, true);
+  else if (p.C <= 16) ENS_LAUNCH(16, false);
+  else ENS_LAUNCH(32, false);
+#undef ENS_LAUNCH
+}
+
+KDCC_API int kdcc_ensemble_loss(const void *s, const void *const *teachers, const float *kd_weights, int K, float T,
+                                const long long *labels, const float *class_weight, int ignore_index, int mean,
+                                void *ds, float *out3, long long *bad_labels, void *workspace, size_t workspace_bytes,
+                                int N, int C, long HW, long batch_stride, long class_stride, long pixel_stride, int dtype,
+                                float kd_grad_scale, float ce_grad_scale, const float *upstream2, kdcc_stream_t stream) {
+  int rc = ce_args(N, C, HW, dtype);
+  if (rc) return rc;
+  if (K < 1 || K > kEnsMaxTeachers || !(T > 0.f)) return KDCC_EINVAL;
+  if (!s || !teachers || !kd_weights || !labels || !out3 || !workspace || (upstream2 && !ds)) return KDCC_EINVAL;
+  for (int k = 0; k < K; ++k)
+    if (!teachers[k]) return KDCC_EINVAL;
+  if (workspace_bytes < kdcc_ce_workspace_bytes(N, HW)) return KDCC_EWORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  EnsParams p{};
+  p.s = s; p.K = K; p.labels = labels; p.weight = class_weight; p.ds = ds;
+  double wsum = 0.0;
+  bool vec2 = ce_vec2(s, nullptr, ds, labels, HW, batch_stride, class_stride, pixel_stride, dtype) && C == 10;
+  const uintptr_t va = dtype == KDCC_F32 ? 8 : 4;
+  for (int k = 0; k < K; ++k) {
+    p.t[k] = teachers[k];
+    p.w[k] = kd_weights[k];
+    wsum += kd_weights[k];
+    vec2 = vec2 && (uintptr_t)teachers[k] % va == 0;
+  }
+  p.wsum = (float)wsum;
+  p.part = static_cast<float *>(workspace);
+  p.stride = ce_blocks(N, HW);
+  p.bad = reinterpret_cast<unsigned long long *>(bad_labels);
+  p.e_kd = kd_grad_scale; p.e_ce = ce_grad_scale;
+  p.HW = HW; p.bs = batch_stride; p.cs = class_stride; p.ps = pixel_stride;
+  p.C = C; p.ignore = ignore_index;
+  p.shared = T == 1.f;
+  p.k2 = kLog2e / T;
+  p.kd_g = (float)((double)T / ((double)N * (double)HW));
+  p.HWg = vec2 ? HW / 2 : HW;
+  p.groups = (long)N * p.HWg;
+  const int grid = (int)min(p.stride, ceil_div<long>(p.groups, kLossThreads));
+  const bool f32 = dtype == KDCC_F32;
+  if (upstream2 != nullptr) {
+    // gradient-only re-launch for the upstream pair autograd actually handed over; D is the one the forward used
+    p.up2 = upstream2;
+    p.den = out3 + 2;
+    p.part = nullptr;
+    p.bad = nullptr;
+    if (f32) launch_ensemble<float, true>(p, vec2, grid, st);
+    else launch_ensemble<__nv_bfloat16, true>(p, vec2, grid, st);
+    return launch_status();
+  }
+  const bool pre = ds != nullptr && mean;
+  if (pre) {
+    // D = sum_valid w from one read of the labels, so that the main pass writes ds once, already normalised
+    ce_weight_sum_kernel<<<(int)p.stride, kLossThreads, 0, st>>>(labels, class_weight, (long)N * HW, C, ignore_index,
+                                                                 p.part + kSlotPre * p.stride);
+    if ((rc = launch_status())) return rc;
+    CeFinal f{};
+    f.part = p.part; f.stride = p.stride; f.count = (int)p.stride; f.mode = 3; f.slots = 1u << kSlotPre;
+    f.out = out3 + 2;
+    launch_pdl(ce_finalize_kernel, dim3(1), dim3(256), 0, st, f);
+    if ((rc = launch_status())) return rc;
+    p.den = out3 + 2;
+  }
+  if (ds != nullptr) {
+    if (f32) launch_ensemble<float, true>(p, vec2, grid, st);
+    else launch_ensemble<__nv_bfloat16, true>(p, vec2, grid, st);
+  } else {
+    if (f32) launch_ensemble<float, false>(p, vec2, grid, st);
+    else launch_ensemble<__nv_bfloat16, false>(p, vec2, grid, st);
+  }
+  if ((rc = launch_status())) return rc;
+  CeFinal f{};
+  f.part = p.part; f.stride = p.stride; f.count = grid; f.mode = 4; f.mean = mean; f.out = out3;
+  f.slots = (1u << kSlotCeS) | (1u << kSlotW) | (1u << kSlotKd);
+  f.den_done = pre;   // keep the D the gradient was formed with
+  f.kd_coef = (double)kLn2 * (double)T * (double)T / ((double)N * (double)HW);
   launch_pdl(ce_finalize_kernel, dim3(1), dim3(256), 0, st, f);
   return launch_status();
 }

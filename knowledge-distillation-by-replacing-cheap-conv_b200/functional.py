@@ -11,6 +11,7 @@ Reference call sites replaced (reference file:line):
   hint_loss           losses/WeightedHintMSELoss.py:12-16, losses/MSELoss.py:14-16
   cross_entropy       losses/CrossEntropy.py:10-15
   logits_stats        trainer/layerwise_trainer.py:225-227,244-250 (logged losses + confusion matrices, one pass)
+  ensemble_loss       trainer/ensemble_trainer.py:73-90 (kd + supervised and their summed gradient, one pass)
 """
 import os
 
@@ -589,6 +590,71 @@ def cross_entropy(logits, target, weight=None, ignore_index=255, mean=True, expe
     dropped, never used as an index, and added to `bad_labels` (one-element int64 device tensor) when given.
     `expected_upstream`: see kd_loss."""
     return _CeLoss.apply(logits, target, weight, int(ignore_index), bool(mean), float(expected_upstream), bad_labels)
+
+
+class _EnsembleLoss(torch.autograd.Function):
+    @staticmethod
+    @_device_guard
+    def forward(ctx, s, target, class_weight, ignore_index, mean, temperature, kd_weights, expected, bad_labels, *teachers):
+        import ctypes
+        _require_cuda(s, target, class_weight, bad_labels, *teachers)
+        K = len(teachers)
+        if not 1 <= K <= 8 or K != len(kd_weights):
+            raise _abi.KdccError("ensemble_loss needs 1 to 8 teachers and one weight each (got %d teachers, %d weights)"
+                                 % (K, len(kd_weights)))
+        for t in teachers:
+            if t.shape != s.shape:
+                raise _abi.KdccError("ensemble_loss expects matching (N, C, ...) tensors, got %s and %s" % (tuple(s.shape), tuple(t.shape)))
+        s, target, w, geo = _ce_operands(s, target, class_weight, bad_labels)
+        fmt = torch.channels_last if geo[5] != 1 else torch.contiguous_format
+        ts = [t.detach().to(s.dtype).contiguous(memory_format=fmt) for t in teachers]
+        ds = torch.empty_like(s) if ctx.needs_input_grad[0] else None
+        out3 = torch.empty(3, dtype=torch.float32, device=s.device)
+        ctx.call = (s, ts, (ctypes.c_float * K)(*[float(x) for x in kd_weights]), float(temperature), target, w,
+                    int(ignore_index), int(bool(mean)), geo, (float(expected[0]), float(expected[1])))
+        _EnsembleLoss._launch(ctx.call, ds, out3, bad_labels, None)
+        # forward wrote ds for the expected upstream pair; backward re-launches only for the gradient, reading D from out3
+        ctx.ds, ctx.out3 = ds, out3
+        return out3[0], out3[1]
+
+    @staticmethod
+    def _launch(call, ds, out3, bad_labels, upstream2):
+        import ctypes
+        s, ts, wts, T, target, w, ignore, mean, (N, C, HW, bs, cs, ps), (e_kd, e_ce) = call
+        L = _abi.lib()
+        ws = _workspace(L.kdcc_ce_workspace_bytes(N, HW), s.device)
+        ptrs = (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+        _abi.check(L.kdcc_ensemble_loss(_ptr(s), ptrs, wts, len(ts), T, _ptr(target), _ptr(w), ignore, mean, _ptr(ds),
+                                        _ptr(out3), _ptr(bad_labels), _ptr(ws), ws.numel(), N, C, HW, bs, cs, ps,
+                                        _dtype_code(s), e_kd, e_ce, _ptr(upstream2), _stream()), "kdcc_ensemble_loss")
+
+    @staticmethod
+    @_device_guard
+    def backward(ctx, g_kd, g_ce):
+        ds = _take_grad(ctx)
+        nones = (None,) * (8 + len(ctx.call[1]))
+        if ds is None:
+            return (None,) + nones
+        up2 = torch.stack((g_kd.detach().float().reshape(()), g_ce.detach().float().reshape(())))
+        _EnsembleLoss._launch(ctx.call, ds, ctx.out3, None, up2)
+        ctx.call = None
+        return (ds,) + nones
+
+
+def ensemble_loss(inputs, teachers, kd_weights, target, class_weight=None, ignore_index=255, mean=True, temperature=1.0,
+                  expected_upstream=(1.0, 1.0), bad_labels=None):
+    """The objective of trainer/ensemble_trainer.py:73-90 in one pass over the student logits: returns (kd, ce), two fp32
+    0-dim tensors of ONE autograd node, where
+      kd = kd_loss_multi(inputs, teachers, kd_weights, temperature)
+      ce = cross_entropy(inputs, target, class_weight, ignore_index, mean, bad_labels=bad_labels)
+    The student logits, every teacher and the labels are read once and d(kd)/d(inputs) + d(ce)/d(inputs) is written once.
+    `expected_upstream`: the (kd, ce) pair autograd is expected to hand to backward ((1/acc, 1/acc) for
+    `(kd + ce) / acc`); it is folded into that gradient, and backward re-forms the gradient in one more pass only when
+    the actual pair differs -- a performance hint, never a correctness assumption."""
+    teachers = list(teachers)
+    e = tuple(float(x) for x in expected_upstream)
+    return _EnsembleLoss.apply(inputs, target, class_weight, int(ignore_index), bool(mean), float(temperature),
+                               tuple(float(x) for x in kd_weights), e, bad_labels, *teachers)
 
 
 def _conf_arg(conf, C):

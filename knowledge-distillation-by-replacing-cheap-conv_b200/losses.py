@@ -103,3 +103,33 @@ class MultiTeacherKLDivergenceLoss(nn.Module):
             w.append(1.0)
         total = sum(w)
         return F_kdcc.kd_loss_multi(inputs, outs, [x / total for x in w], self.temperature, expected_upstream=self.expected_upstream)
+
+
+class EnsembleDistillationLoss(nn.Module):
+    """The whole objective of trainer/ensemble_trainer.py:73-90 as one module: forward(inputs, ensemble_outputs,
+    teacher_output, targets) returns (kd, supervised), equal to
+        (MultiTeacherKLDivergenceLoss(temperature, weight)(inputs, ensemble_outputs, teacher_output),
+         CrossEntropyLoss2d(class_weight, size_average, ignore_index)(inputs, targets))
+    from ONE pass over the student logits (kdcc_ensemble_loss): every teacher and the labels are read once and the
+    gradient of kd + supervised is written once.  `expected_upstream` is the (kd, supervised) pair of upstream values
+    backward expects (kdcc.EnsembleStep sets (1/acc, 1/acc)); an unexpected pair costs one more pass, never correctness."""
+
+    def __init__(self, temperature=1, weight=1, class_weight=None, size_average=True, ignore_index=255):
+        super().__init__()
+        self.temperature = temperature
+        self.weight = weight  # WEIGHT of trainer/ensemble_trainer.py:10
+        self.register_buffer("class_weight", class_weight)
+        self.size_average = size_average
+        self.ignore_index = ignore_index
+        self.expected_upstream = (1.0, 1.0)
+
+    def forward(self, inputs, ensemble_outputs, teacher_output, targets):
+        outs = list(ensemble_outputs)
+        w = [float(self.weight)] * len(outs)
+        if teacher_output is not None:
+            outs.append(teacher_output)
+            w.append(1.0)
+        total = sum(w)
+        return F_kdcc.ensemble_loss(inputs, outs, [x / total for x in w], targets, self.class_weight, self.ignore_index,
+                                    mean=self.size_average is not False, temperature=self.temperature,
+                                    expected_upstream=self.expected_upstream)

@@ -243,14 +243,21 @@ class EnsembleStep:
         kd = (sum_k WEIGHT * crit_kd(student, model_k(x)) + crit_kd(student, teacher)) / (WEIGHT * K + 1)
     and `loss = kd + supervised`, both divided by accumulation_steps; step on `(batch_idx + 1) % accumulation_steps`.
     `kd_multi` (a kdcc.MultiTeacherKLDivergenceLoss) computes the whole KD term in one fused pass -- student logits read
-    once, every teacher once; without it the term is composed from criterions[1] exactly as the reference composes it."""
+    once, every teacher once; without it the term is composed from criterions[1] exactly as the reference composes it.
+    `objective` (a kdcc.EnsembleDistillationLoss) gives kd and supervised from ONE pass over the student logits and
+    writes the gradient of their sum once; criterions and kd_multi are then unused."""
 
-    def __init__(self, model, models, criterions, optimizer, accumulation_steps=1, weight=1, kd_multi=None, process_group=None):
+    def __init__(self, model, models, criterions, optimizer, accumulation_steps=1, weight=1, kd_multi=None, process_group=None,
+                 objective=None):
         self.model, self.models, self.criterions, self.optimizer = model, list(models), criterions, optimizer
         self.accumulation_steps, self.weight, self.kd_multi = int(accumulation_steps), weight, kd_multi
+        self.objective = objective
         self.group = process_group
         self.bucket = GradBucket(model.trainable_parameters())
-        _expect(criterions[0], 1.0 / self.accumulation_steps)   # loss = kd + supervised / accumulation_steps
+        if objective is not None:
+            objective.expected_upstream = (1.0 / self.accumulation_steps,) * 2   # loss = (kd + supervised) / acc
+        else:
+            _expect(criterions[0], 1.0 / self.accumulation_steps)   # loss = kd + supervised / accumulation_steps
 
     def rebuild_bucket(self):
         self.bucket = GradBucket(self.model.trainable_parameters())
@@ -260,12 +267,19 @@ class EnsembleStep:
         output_st, output_tc = self.model(data)
         with torch.no_grad():
             outputs = [m(data) for m in self.models]
+        if self.objective is not None:
+            kd_loss, supervised = self.objective(output_st, outputs, output_tc, target)
+            return self._finish(kd_loss / acc, supervised / acc, output_st, output_tc, batch_idx)
         supervised = self.criterions[0](output_st, target) / acc
         if self.kd_multi is not None:
             kd_loss = self.kd_multi(output_st, outputs, output_tc) / acc
         else:
             kd_loss = reduce(lambda a, o: a + self.weight * self.criterions[1](output_st, o), outputs, 0)
             kd_loss = (kd_loss + self.criterions[1](output_st, output_tc)) / (self.weight * len(outputs) + 1) / acc
+        return self._finish(kd_loss, supervised, output_st, output_tc, batch_idx)
+
+    def _finish(self, kd_loss, supervised, output_st, output_tc, batch_idx):
+        acc = self.accumulation_steps
         loss = kd_loss + supervised
         loss.backward()
         if (batch_idx + 1) % acc == 0:
