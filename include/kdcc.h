@@ -246,6 +246,16 @@ int kdcc_tta_stitch(const float *windows, const int *coords, int n, int C, int t
 int kdcc_resize_bilinear(const float *src, int C, int h, int w, float *dst, int H, int W, float alpha, int accumulate,
                          kdcc_stream_t stream);
 
+/* ---- Canny edge map of the Gated-SCNN shape stream (DESIGN.md 4.3f) ---------------------------------------------
+ * kdcc_canny replaces the host round trip of models/gscnn/gscnn.py:284-288 (numpy astype(uint8) + cv2.Canny(img, low,
+ * high) per image + copy back) with a bit-identical device computation: img (N, 3, H, W) fp32 or bf16 in `layout` (NCHW or
+ * NHWC = channels_last), edges fp32 [N][H][W] of 0.f / 255.f.  The cast is numpy's (truncate to int32, low 8 bits; NaN,
+ * +-inf and out-of-int32 values -> 0); then cv2's aperture-3 L1 Canny (reversed thresholds swapped, both floored).  Four
+ * launches whatever the content, no host synchronisation.  C != 3 or N*H*W >= 2^31: KDCC_ESHAPE. */
+size_t kdcc_canny_workspace_bytes(int N, int H, int W);
+int kdcc_canny(const void *img, float *edges, void *workspace, size_t workspace_bytes, int N, int C, int H, int W,
+               int layout, int dtype, double low, double high, kdcc_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -50,6 +50,8 @@ SIGNATURES = {
     "kdcc_radam_step_multi": (_i, [_vp, _vp, _l, _i, _vp, _vp, _vp, _l, _f, _f, _f, _f, _f, _f, _f, _i, _vp]),
     "kdcc_tta_stitch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _f, _vp, _i, _vp]),
     "kdcc_resize_bilinear": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _f, _i, _vp]),
+    "kdcc_canny_workspace_bytes": (_sz, [_i, _i, _i]),
+    "kdcc_canny": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _i, ctypes.c_double, ctypes.c_double, _vp]),
 }
 
 _lib = None

@@ -12,6 +12,7 @@ Reference call sites replaced (reference file:line):
   cross_entropy       losses/CrossEntropy.py:10-15
   logits_stats        trainer/layerwise_trainer.py:225-227,244-250 (logged losses + confusion matrices, one pass)
   ensemble_loss       trainer/ensemble_trainer.py:73-90 (kd + supervised and their summed gradient, one pass)
+  canny_edges         models/gscnn/gscnn.py:284-288 (uint8 cast + cv2.Canny per image, without the host round trip)
 """
 import os
 
@@ -762,3 +763,33 @@ def resize_bilinear(src, out, alpha=1.0, accumulate=False):
     _abi.check(_abi.lib().kdcc_resize_bilinear(_ptr(src), C, h, w, _ptr(out), out.shape[1], out.shape[2], float(alpha),
                                                int(bool(accumulate)), _stream()), "kdcc_resize_bilinear")
     return out
+
+
+# ---------------------------------------------------------------------------------------------------
+# Canny edge map of the Gated-SCNN shape stream (DESIGN.md 4.3f)
+# ---------------------------------------------------------------------------------------------------
+@torch.no_grad()
+@_device_guard
+def canny_edges(inp, low_threshold=10, high_threshold=100):
+    """(N, 1, H, W) fp32 map of 0.0 / 255.0, bit-identical to models/gscnn/gscnn.py:284-288:
+        im = inp.cpu().numpy().transpose((0, 2, 3, 1)).astype(np.uint8)
+        canny[i] = cv2.Canny(im[i], low_threshold, high_threshold)   # aperture 3, L1 gradient
+    computed on the device and on the current stream, with no host synchronisation.  `inp` is (N, 3, H, W) fp32 or bf16
+    (bf16 is widened exactly), NCHW-contiguous or channels_last."""
+    _require_cuda(inp)
+    if inp.dim() != 4 or inp.shape[1] != 3:
+        raise _abi.KdccError("canny_edges expects an (N, 3, H, W) image, got %s" % (tuple(inp.shape),))
+    code = _dtype_code(inp)
+    if inp.is_contiguous():
+        layout = _abi.NCHW
+    elif inp.is_contiguous(memory_format=torch.channels_last):
+        layout = _abi.NHWC
+    else:
+        inp, layout = inp.contiguous(), _abi.NCHW
+    N, C, H, W = inp.shape
+    edges = torch.empty((N, 1, H, W), dtype=torch.float32, device=inp.device)
+    L = _abi.lib()
+    ws = _workspace(L.kdcc_canny_workspace_bytes(N, H, W), inp.device)
+    _abi.check(L.kdcc_canny(_ptr(inp), _ptr(edges), _ptr(ws), ws.numel(), N, C, H, W, layout, code, float(low_threshold),
+                            float(high_threshold), _stream()), "kdcc_canny")
+    return edges
