@@ -17,6 +17,10 @@
  *     layouts dispatch to different kernels (NCHW bf16 depthwise runs on the tensor cores); logits carry
  *     explicit strides;
  *   - dtype: KDCC_F32 (parity path, 1e-5 relative) or KDCC_BF16 (production path, fp32 accumulate);
+ *     KDCC_F32_TF32X3 (pointwise entry points only, NHWC only): fp32 tensors whose products are formed as three tf32
+ *     tensor-core MMAs (hi.hi + hi.lo + lo.hi of x = hi + lo), within the fp32 parity tolerance; shapes the tensor-core
+ *     kernel does not take (K or Nc % 4 != 0) run on the CUDA-core fp32 kernel; every other entry point returns
+ *     KDCC_EINVAL for it;
  *   - return 0 on success, a negative KDCC_E* code for bad arguments / unsupported shapes (there is
  *     NO CPU or library fallback), or a positive cudaError_t.  kdcc_strerror() names any of them.
  */
@@ -32,7 +36,7 @@ extern "C" {
 
 #define KDCC_VERSION 104 /* round 1: layout-aware depthwise/pointwise, confusion matrix, multi-teacher KD, TTA stitch, RAdam */
 
-enum { KDCC_F32 = 0, KDCC_BF16 = 1 };
+enum { KDCC_F32 = 0, KDCC_BF16 = 1, KDCC_F32_TF32X3 = 2 };
 enum { KDCC_LAYOUT_NHWC = 0, KDCC_LAYOUT_NCHW = 1,
        /* pointwise entry points only: the block-INTERNAL tensor (depthwise output `x`, its gradient `dx`) is channel planes
         * (NCHW), the block-EXTERNAL one (`y`, `dy`) is channels_last -- a block whose depthwise ran on planes inside a
@@ -82,6 +86,8 @@ int kdcc_dw_bwd(const void *x, const float *w, const void *dy, void *dx, float *
  * w [Nc,K] in the activation dtype (the (Co,C,1,1) parameter, cast by kdcc_cast_f32_to_bf16).
  * layout NHWC: x [M,K], out [M,Nc], out[m][n] = sum_k x[m][k] w[n][k]  (batch ignored);
  * layout NCHW: x [batch,K,M/batch], out [batch,Nc,M/batch], out_b = W . x_b  (bf16 tensor-core path only).
+ * dtype KDCC_F32_TF32X3: fp32 tensors, NHWC only (any other layout: KDCC_ESHAPE); K % 4 == 0 and Nc % 4 == 0 run on the
+ * tensor cores (16-byte aligned pointers, else KDCC_EALIGN), other shapes on the CUDA-core fp32 kernel.
  * Optional fused epilogue on the second output:
  *   y_act = relu?( out * scale[n] + shift[n] )   (eval-mode BN fold + ReLU, SURVEY.md F9;
  *   scale NULL -> 1, shift NULL -> 0; shift alone is the conv bias).

@@ -10,6 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KDCC_LIB", os.path.join(_HERE, "libkdcc.so"))  # KDCC_LIB: A/B builds of the same library (tools/)
 
 F32, BF16 = 0, 1
+F32_TF32X3 = 2   # pointwise only: fp32 tensors, products as three tf32 tensor-core MMAs
 NHWC, NCHW = 0, 1
 PLANES_TO_NHWC = 2   # pointwise only: input / input-gradient as channel planes, output / output-gradient channels_last
 

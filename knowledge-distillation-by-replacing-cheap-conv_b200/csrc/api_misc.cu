@@ -38,6 +38,12 @@ KDCC_API const char *kdcc_dispatch_name(int op, int N, int H, int W, int C, int 
   const long M = (long)N * H * W;
   const int Ho = H + 2 * pad - dil * (k - 1), Wo = W + 2 * pad - dil * (k - 1);
   const bool nchw = layout == KDCC_LAYOUT_NCHW;
+  if (dtype == KDCC_F32_TF32X3) {
+    // pointwise, NHWC only: the tf32x3 kernel, or the CUDA-core fp32 kernel for the shapes it does not take
+    static const char *names[3] = {"pw_tf32x3_fwd", "pw_tf32x3_dx", "pw_tf32x3_dw"};
+    if (op < 2 || op > 4 || layout != KDCC_LAYOUT_NHWC) return "unsupported";
+    return pw_tf32x3_supported(M, C, Cout) ? names[op - 2] : "pw_simt";
+  }
   switch (op) {
     case 0:
       if (nchw) return bf16 && dw_tc_supported(H, W, Ho, Wo, k, dil) ? "dw_tc_conv" : "unsupported";

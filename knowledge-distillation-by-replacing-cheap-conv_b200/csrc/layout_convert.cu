@@ -97,6 +97,7 @@ using namespace kdcc;
 // dst (NCHW if to_nchw else NHWC) = src (the other layout); bf16; C % 8 == 0 and HW % 8 == 0 (16-byte rows both ways)
 KDCC_API int kdcc_layout_convert(const void *src, void *dst, int N, int C, long HW, int to_nchw, int dtype, kdcc_stream_t stream) {
   if (!src || !dst || N < 0 || C <= 0 || HW <= 0) return KDCC_EINVAL;
+  if (dtype == KDCC_F32_TF32X3) return KDCC_EINVAL;  // a pointwise-only dtype code
   if (dtype != KDCC_BF16) return KDCC_ESHAPE;
   if (C % 8 != 0 || HW % 8 != 0) return KDCC_ESHAPE;
   if (!aligned16(src) || !aligned16(dst)) return KDCC_EALIGN;

@@ -650,7 +650,7 @@ KDCC_API int kdcc_cast_f32_to_bf16(const float *src, void *dst, long n, kdcc_str
 }
 
 KDCC_API int kdcc_scale_inplace_expect(void *buf, const float *dev_scalar, float expected, long n, int dtype, kdcc_stream_t stream) {
-  if (!buf || !dev_scalar || n < 0 || !(expected != 0.f)) return KDCC_EINVAL;
+  if (!buf || !dev_scalar || n < 0 || !(expected != 0.f) || (dtype != KDCC_F32 && dtype != KDCC_BF16)) return KDCC_EINVAL;
   if (n == 0) return KDCC_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int grid = (int)min((long)kNumSMs * 8, ceil_div<long>(n, 256 * 8));

@@ -15,6 +15,14 @@ int pw_sm100_bwd_dw(const void *dy, const void *x, float *dw, float *part, long 
                     cudaStream_t st);
 __global__ void reduce_splits_kernel(const float *__restrict__ part, float *__restrict__ out, int splits, long count);
 
+// ---- fp32 as three tf32 tcgen05 products (KDCC_F32_TF32X3): pw_gemm_tf32x3.cu, NHWC only ---------------
+bool pw_tf32x3_supported(long M, int K, int Nc);
+int pw_tf32x3_fwd(const void *x, const void *w, const float *scale, const float *shift, const void *residual, int relu,
+                  void *y_raw, void *y_act, long M, int K, int Nc, cudaStream_t st);
+int pw_tf32x3_bwd_dx(const void *dy, const void *w, void *dx, long M, int K, int Nc, cudaStream_t st);
+int pw_tf32x3_dw_splits(long M, int K, int Nc);
+int pw_tf32x3_bwd_dw(const void *dy, const void *x, float *dw, float *part, long M, int K, int Nc, cudaStream_t st);
+
 // ---- CUDA-core GEMM (fp32 parity path, shapes the tensor-core kernel does not take): pw_gemm_simt.cu -
 // C[i][j] = sum_r A[i*sai + r*sar] * B[j*sbj + r*sbr]
 struct SimtGemm {

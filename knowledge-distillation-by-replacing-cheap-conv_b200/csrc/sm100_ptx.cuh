@@ -118,6 +118,24 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint6
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem desc] * B[smem desc], fp32 operands read as tf32, fp32 accumulate
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
+      "}\n"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// x rounded to the nearest tf32 value (ties away from zero), as an fp32 bit pattern with the low 13 bits clear
+__device__ __forceinline__ float cvt_rna_tf32(float x) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return __uint_as_float(r);
+}
 // mbarrier arrives once every previously issued tcgen05.mma of this thread has completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -292,6 +310,9 @@ EncodeTiledFn get_encode_tiled();  // nullptr when the driver cannot provide it
 // rank-`rank` tiled map over a bf16 tensor; dims/strides innermost first, strides in BYTES for dims 1..rank-1
 int make_tmap_bf16(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides_bytes,
                    const uint32_t *box, const uint32_t *elem_strides, CUtensorMapSwizzle swizzle);
+// the same over an fp32 tensor
+int make_tmap_f32(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides_bytes,
+                  const uint32_t *box, const uint32_t *elem_strides, CUtensorMapSwizzle swizzle);
 
 int last_driver_status();  // CUresult of this thread's last descriptor encode (diagnostics)
 

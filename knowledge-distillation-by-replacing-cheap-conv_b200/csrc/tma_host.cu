@@ -26,8 +26,9 @@ EncodeTiledFn get_encode_tiled() {
   return fn;
 }
 
-int make_tmap_bf16(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides_bytes,
-                   const uint32_t *box, const uint32_t *elem_strides, CUtensorMapSwizzle swizzle) {
+static int make_tmap(CUtensorMapDataType type, CUtensorMap *out, const void *base, int rank, const uint64_t *dims,
+                     const uint64_t *strides_bytes, const uint32_t *box, const uint32_t *elem_strides,
+                     CUtensorMapSwizzle swizzle) {
   EncodeTiledFn enc = get_encode_tiled();
   if (!enc) return KDCC_EDEVICE;
   // The encoder is a driver-API call and needs a current context on THIS thread.  Autograd runs backward
@@ -46,11 +47,21 @@ int make_tmap_bf16(CUtensorMap *out, const void *base, int rank, const uint64_t 
     estr[i] = elem_strides ? elem_strides[i] : 1;
     if (i > 0) gstr[i - 1] = strides_bytes[i - 1];
   }
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(base), gdim, gstr, bdim,
+  CUresult r = enc(out, type, (cuuint32_t)rank, const_cast<void *>(base), gdim, gstr, bdim,
                    estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   g_last_driver_status = (int)r;
   return r == CUDA_SUCCESS ? KDCC_OK : KDCC_ESHAPE;
+}
+
+int make_tmap_bf16(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides_bytes,
+                   const uint32_t *box, const uint32_t *elem_strides, CUtensorMapSwizzle swizzle) {
+  return make_tmap(CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, out, base, rank, dims, strides_bytes, box, elem_strides, swizzle);
+}
+
+int make_tmap_f32(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides_bytes,
+                  const uint32_t *box, const uint32_t *elem_strides, CUtensorMapSwizzle swizzle) {
+  return make_tmap(CU_TENSOR_MAP_DATA_TYPE_FLOAT32, out, base, rank, dims, strides_bytes, box, elem_strides, swizzle);
 }
 
 int last_driver_status() { return g_last_driver_status; }

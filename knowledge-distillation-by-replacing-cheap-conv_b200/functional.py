@@ -259,6 +259,15 @@ def depthwise_conv(x, weight, bias, kernel_size, dilation, padding):
 # ---------------------------------------------------------------------------------------------------
 # pointwise
 # ---------------------------------------------------------------------------------------------------
+def _pw_code(x):
+    """dtype code of a pointwise GEMM: fp32 runs as three tf32 tensor-core products (fp32 accuracy) unless torch's float32
+    matmul precision is "highest", its default, under which the products are plain fp32 FMAs."""
+    code = _dtype_code(x)
+    if code == _abi.F32 and torch.get_float32_matmul_precision() != "highest":
+        return _abi.F32_TF32X3
+    return code
+
+
 class _PointwiseConv(torch.autograd.Function):
     @staticmethod
     @_device_guard
@@ -275,6 +284,7 @@ class _PointwiseConv(torch.autograd.Function):
             if out_channels_last and Co % 8 == 0 and _supported(2, N, H, W, K, Co, 1, 1, 0, _abi.PLANES_TO_NHWC, code):
                 layout = _abi.PLANES_TO_NHWC
         x = _format(x, _abi.NCHW if layout == _abi.PLANES_TO_NHWC else layout)
+        pw_code = _pw_code(x) if layout == _abi.NHWC else code
         w = lp_weight(weight, x.dtype).reshape(Co, K)
         y = _empty_like_layout(N, Co, H, W, x, _abi.NHWC if layout == _abi.PLANES_TO_NHWC else layout)
         fused = scale is not None or shift is not None or relu
@@ -289,17 +299,18 @@ class _PointwiseConv(torch.autograd.Function):
                 raise _abi.KdccError("residual %s does not match the output %s" % (tuple(residual.shape), tuple(y.shape)))
             res = _format(residual.detach().to(x.dtype), _abi.NHWC if layout == _abi.PLANES_TO_NHWC else layout)
             _abi.check(_abi.lib().kdcc_pw_fwd_residual(_ptr(x), _ptr(w), _ptr(scale), _ptr(eff_shift), _ptr(res), int(bool(relu)),
-                                                       None, _ptr(y), M, K, Co, N, layout, code, _stream()), "kdcc_pw_fwd_residual")
+                                                       None, _ptr(y), M, K, Co, N, layout, pw_code, _stream()), "kdcc_pw_fwd_residual")
         else:
             _abi.check(_abi.lib().kdcc_pw_fwd(_ptr(x), _ptr(w), _ptr(scale), _ptr(eff_shift), int(bool(relu)),
                                               None if use_act else _ptr(y), _ptr(y) if use_act else None,
-                                              M, K, Co, N, layout, code, _stream()), "kdcc_pw_fwd")
+                                              M, K, Co, N, layout, pw_code, _stream()), "kdcc_pw_fwd")
         if out_channels_last and layout == _abi.NCHW and _convertible(y):
             y = _convert(y, False)          # hand the result back in the caller's (channels_last) layout
         if fused:
             ctx.mark_non_differentiable(y)  # inference-only epilogue (eval-mode BN fold)
         ctx.save_for_backward(x, w)
         ctx.meta = (bias is not None, weight.shape, layout)
+        ctx.pw_code = pw_code   # backward keeps the forward's choice even if the precision setting changes in between
         ctx.wdtype = weight.dtype
         ctx.has_residual = residual is not None
         return y
@@ -316,15 +327,16 @@ class _PointwiseConv(torch.autograd.Function):
         dy = _format(dy, _abi.NHWC if mixed else layout)
         L = _abi.lib()
         code = _dtype_code(x)
+        pw_code = ctx.pw_code
         st = _stream()
         dx = dw = db = None
         if ctx.needs_input_grad[0]:
             dx = _empty_like_layout(N, K, H, W, x, _abi.NCHW if mixed else layout)
-            _abi.check(L.kdcc_pw_bwd_dx(_ptr(dy), _ptr(w), _ptr(dx), None, 0, M, K, Co, N, layout, code, st), "kdcc_pw_bwd_dx")
+            _abi.check(L.kdcc_pw_bwd_dx(_ptr(dy), _ptr(w), _ptr(dx), None, 0, M, K, Co, N, layout, pw_code, st), "kdcc_pw_bwd_dx")
         if ctx.needs_input_grad[1]:
             dw = torch.empty((Co, K), dtype=torch.float32, device=x.device)
-            ws = _workspace(L.kdcc_pw_bwd_workspace_bytes(1, M, K, Co, code), x.device)
-            _abi.check(L.kdcc_pw_bwd_dw(_ptr(dy), _ptr(x), _ptr(dw), _ptr(ws), ws.numel(), M, K, Co, N, layout, code, st),
+            ws = _workspace(L.kdcc_pw_bwd_workspace_bytes(1, M, K, Co, pw_code), x.device)
+            _abi.check(L.kdcc_pw_bwd_dw(_ptr(dy), _ptr(x), _ptr(dw), _ptr(ws), ws.numel(), M, K, Co, N, layout, pw_code, st),
                        "kdcc_pw_bwd_dw")
             dw = dw.reshape(wshape).to(ctx.wdtype)
         if has_bias and ctx.needs_input_grad[2]:
