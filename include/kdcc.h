@@ -252,6 +252,21 @@ int kdcc_tta_stitch(const float *windows, const int *coords, int n, int C, int t
 int kdcc_resize_bilinear(const float *src, int C, int h, int w, float *dst, int H, int W, float alpha, int accumulate,
                          kdcc_stream_t stream);
 
+/* kdcc_tta_windows replaces the host preparation of utils/tta_process.py:52-117 for one image and one scale (DESIGN.md
+ * 4.3h): ToPILImage (pic.mul(255).byte() in the input dtype), PIL resize to (w, h) BILINEAR, FLIP_LEFT_RIGHT, ToTensor +
+ * Normalize(mean m0..m2, std s0..s2) and the window crops, bit-identical to that host computation.  img (3, H, W) fp32
+ * (dtype KDCC_F32) or bf16 (KDCC_BF16) on the device, NCHW-contiguous.  out fp32 [2n][3][th][tw], th = min(tile, h),
+ * tw = min(tile, w): the n windows of tta.window_coordinates (x outer / y inner, n = nx * ny with
+ * nx = ceil((w - tile) / stride) + 1, likewise ny; no window when either is < 1), then the same n windows of the mirrored
+ * image.  Up to three launches, no host synchronisation.  The workspace may be NULL when
+ * kdcc_tta_windows_workspace_bytes returns 0 (h == H and w == W).  Null img / out, non-positive sizes, tile or stride
+ * < 1, dtype other than KDCC_F32 / KDCC_BF16: KDCC_EINVAL; image, intermediate or output of 2^31 elements or more:
+ * KDCC_ESHAPE. */
+size_t kdcc_tta_windows_workspace_bytes(int H, int W, int h, int w);
+int kdcc_tta_windows(const void *img, int H, int W, int dtype, int h, int w, int tile, int stride, float m0, float m1,
+                     float m2, float s0, float s1, float s2, float *out, void *workspace, size_t workspace_bytes,
+                     kdcc_stream_t stream);
+
 /* ---- Canny edge map of the Gated-SCNN shape stream (DESIGN.md 4.3f) ---------------------------------------------
  * kdcc_canny replaces the host round trip of models/gscnn/gscnn.py:284-288 (numpy astype(uint8) + cv2.Canny(img, low,
  * high) per image + copy back) with a bit-identical device computation: img (N, 3, H, W) fp32 or bf16 in `layout` (NCHW or

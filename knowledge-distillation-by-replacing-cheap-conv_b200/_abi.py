@@ -51,6 +51,8 @@ SIGNATURES = {
     "kdcc_radam_step_multi": (_i, [_vp, _vp, _l, _i, _vp, _vp, _vp, _l, _f, _f, _f, _f, _f, _f, _f, _i, _vp]),
     "kdcc_tta_stitch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _f, _vp, _i, _vp]),
     "kdcc_resize_bilinear": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _f, _i, _vp]),
+    "kdcc_tta_windows_workspace_bytes": (_sz, [_i] * 4),
+    "kdcc_tta_windows": (_i, [_vp] + [_i] * 7 + [_f] * 6 + [_vp, _vp, _sz, _vp]),
     "kdcc_canny_workspace_bytes": (_sz, [_i, _i, _i]),
     "kdcc_canny": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _i, ctypes.c_double, ctypes.c_double, _vp]),
 }

@@ -30,12 +30,6 @@ constexpr int CANNY_RH = CANNY_TH + 2, CANNY_RW = CANNY_TW + 2;  // magnitudes: 
 constexpr int CANNY_TG22 = 13573;                                // round(tan(22.5 deg) * 2^15), as cv2
 constexpr int CANNY_PERIM = CANNY_TW + 2 * (CANNY_TH - 1);       // top row + left and right columns below it
 
-// numpy's float -> uint8 on x86-64: cvttss2si to int32 (out of range / NaN -> INT_MIN, whose low byte is 0), low byte
-__device__ __forceinline__ uint8_t cast_u8_like_numpy(float v) {
-  const float t = truncf(v);
-  return (t >= -2147483648.f && t < 2147483648.f) ? (uint8_t)(int)t : (uint8_t)0;
-}
-
 __device__ __forceinline__ float load_f32(const float *p, long i) { return __ldg(p + i); }
 __device__ __forceinline__ float load_f32(const __nv_bfloat16 *p, long i) { return __bfloat162float(p[i]); }
 

@@ -81,6 +81,13 @@ __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) {
   return __float2bfloat16_rn(v);
 }
 
+// numpy's / torch's float -> uint8 on x86-64: cvttss2si to int32 (out of range / NaN -> INT_MIN, whose low byte is 0),
+// low byte.  PTX cvt.rzi saturates instead, hence the explicit range check.
+__device__ __forceinline__ uint8_t cast_u8_like_numpy(float v) {
+  const float t = truncf(v);
+  return (t >= -2147483648.f && t < 2147483648.f) ? (uint8_t)(int)t : (uint8_t)0;
+}
+
 // bf16x2 word -> two floats (low element first) with one ALU op each
 __device__ __forceinline__ float bf16lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf16hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }

@@ -13,6 +13,7 @@ Reference call sites replaced (reference file:line):
   logits_stats        trainer/layerwise_trainer.py:225-227,244-250 (logged losses + confusion matrices, one pass)
   ensemble_loss       trainer/ensemble_trainer.py:73-90 (kd + supervised and their summed gradient, one pass)
   canny_edges         models/gscnn/gscnn.py:284-288 (uint8 cast + cv2.Canny per image, without the host round trip)
+  tta_windows         utils/tta_process.py:52-117 (PIL rescale, mirror, normalise and window crops, without the host round trip)
 """
 import os
 
@@ -805,3 +806,49 @@ def canny_edges(inp, low_threshold=10, high_threshold=100):
     _abi.check(L.kdcc_canny(_ptr(inp), _ptr(edges), _ptr(ws), ws.numel(), N, C, H, W, layout, code, float(low_threshold),
                             float(high_threshold), _stream()), "kdcc_canny")
     return edges
+
+
+# ---------------------------------------------------------------------------------------------------
+# Test-time windows of inference_test (DESIGN.md 4.3h)
+# ---------------------------------------------------------------------------------------------------
+def tta_window_count(w, h, tile, stride):
+    """n of tta_windows: nx * ny with nx = ceil((w - tile) / stride) + 1 as tta.window_coordinates counts (0 when the
+    tile overhangs the image by a stride or more)."""
+    nx, ny = (-(-(size - tile) // stride) + 1 for size in (w, h))
+    return nx * ny if nx > 0 and ny > 0 else 0
+
+
+@torch.no_grad()
+@_device_guard
+def tta_windows(img, h, w, tile, stride, mean, std, out=None):
+    """The (2n, 3, th, tw) fp32 window block of one image at one scale, bit-identical to utils/tta_process.py:52-117:
+        image = ToPILImage()(img.cpu())                                # pic.mul(255).byte()
+        scaled = image.resize((w, h), Image.BILINEAR)
+        for im in (scaled, scaled.transpose(Image.FLIP_LEFT_RIGHT)):   # n plain windows, then n mirrored
+            t = Normalize(mean, std)(ToTensor()(im)); windows += [t[:, y1:y2, x1:x2] for the boxes]
+    computed on the device and on the current stream, with no host synchronisation.  img (3, H, W) fp32 or bf16; the
+    boxes are tta.window_coordinates(w, h, tile) with the given stride; (th, tw) = (min(tile, h), min(tile, w)).  `out`
+    (e.g. a slice of a larger batch) receives the block when given."""
+    _require_cuda(img, out)
+    if img.dim() != 3 or img.shape[0] != 3:
+        raise _abi.KdccError("tta_windows expects a (3, H, W) image, got %s" % (tuple(img.shape),))
+    code = _dtype_code(img)
+    img = img.contiguous()
+    _, H, W = img.shape
+    h, w, tile, stride = int(h), int(w), int(tile), int(stride)
+    n = tta_window_count(w, h, tile, stride) if min(h, w, tile, stride) > 0 else 0
+    shape = (2 * n, 3, min(tile, h), min(tile, w))
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float32, device=img.device)
+    elif (out.dtype != torch.float32 or tuple(out.shape) != shape or not out.is_contiguous()
+          or out.device != img.device):
+        raise _abi.KdccError("tta_windows: out must be a contiguous fp32 %s tensor on %s, got %s %s"
+                             % (shape, img.device, out.dtype, tuple(out.shape)))
+    m, s = [float(v) for v in mean], [float(v) for v in std]
+    if len(m) != 3 or len(s) != 3:
+        raise _abi.KdccError("tta_windows needs three means and three standard deviations")
+    L = _abi.lib()
+    ws = _workspace(L.kdcc_tta_windows_workspace_bytes(H, W, h, w), img.device)
+    _abi.check(L.kdcc_tta_windows(_ptr(img), H, W, code, h, w, tile, stride, *m, *s, _ptr(out), _ptr(ws), ws.numel(),
+                                  _stream()), "kdcc_tta_windows")
+    return out

@@ -1,9 +1,10 @@
-"""Sliding-window test-time inference: host mirror of utils/tta_process.py with the stitching on the GPU.
+"""Sliding-window test-time inference on the GPU: window preparation and stitching of utils/tta_process.py.
 
 The reference (models/students/depthwise_student.py:187-206 -> utils/tta_process.py) rescales and mirrors the image
 with PIL, cuts overlapping square windows, runs the student on all of them, copies the outputs to the host and
-stitches them with numpy + cv2 in float64.  Here the preparation keeps the same PIL / torchvision calls (host image
-code is library code), the window outputs never leave the device and `reverse_mapping` is two kdcc kernels
+stitches them with numpy + cv2 in float64.  Here `prepare_windows` makes the windows on the device, bit-identical to
+the PIL / torchvision preparation (`kdcc_tta_windows`; `scale_and_flip_image` / `get_crops_image` keep the host
+formulation as its mirror), the window outputs never leave the device and `reverse_mapping` is two kdcc kernels
 (`kdcc_tta_stitch`, `kdcc_resize_bilinear`).
 
 `count_mode="reference"` reproduces the reference's result exactly -- including its window counter, which
@@ -61,6 +62,37 @@ def get_crops_image(image_data, scales=(1.0,), crop_size=512, overlap=1 / 3):
 
 
 @torch.no_grad()
+def prepare_windows(x, scales, crop_size, mean_std, overlap=1 / 3):
+    """get_crops_image(scale_and_flip_image(ToPILImage()(x.cpu()), mean_std, scales), scales, crop_size) on the device:
+    the same (ori_size, mapping, windows), bit for bit, with `windows` on x's device.  x (3, H, W) fp32 or bf16 CUDA
+    tensor.  Every scale writes its windows straight into one preallocated batch (kdcc_tta_windows); like the
+    reference's torch.cat this needs every scale to give the same window size."""
+    H, W = x.shape[-2:]
+    plan = []
+    for s in scales:
+        w, h, tile = int(W * s), int(H * s), int(s * crop_size)
+        if w < 1 or h < 1:
+            raise ValueError("scale %r makes the %dx%d image empty" % (s, W, H))   # as PIL's resize
+        stride = math.ceil(tile * (1 - overlap))
+        boxes = window_coordinates(w, h, tile, overlap)
+        if not boxes:
+            raise RuntimeError("scale %r gives no window of %d pixels in the %dx%d image" % (s, tile, w, h))  # torch.stack
+        plan.append((w, h, tile, stride, boxes, (min(tile, h), min(tile, w))))
+    for p in plan[1:]:
+        if p[5] != plan[0][5]:
+            raise RuntimeError("Sizes of tensors must match except in dimension 0: scales give %dx%d and %dx%d windows"
+                               % (plan[0][5] + p[5]))   # torch.cat's rule
+    th, tw = plan[0][5]
+    windows = torch.empty((sum(2 * len(p[4]) for p in plan), 3, th, tw), dtype=torch.float32, device=x.device)
+    mapping, at = [], 0
+    for w, h, tile, stride, boxes, _ in plan:
+        F.tta_windows(x, h, w, tile, stride, *mean_std, out=windows[at:at + 2 * len(boxes)])
+        mapping.append([w, h, boxes])
+        at += 2 * len(boxes)
+    return (W, H), mapping, windows
+
+
+@torch.no_grad()
 def reverse_mapping(mapping, results, ori_size, count_mode="reference"):
     """Window outputs -> per-scale class maps at the original size: (n_scales, C, h_ori, w_ori) fp32 on the device
     (utils/tta_process.py:9-26).  results: (total windows, C, th, tw) CUDA tensor in get_crops_image's order."""
@@ -87,14 +119,11 @@ def reverse_mapping(mapping, results, ori_size, count_mode="reference"):
 def inference_test(model, data, args, count_mode="reference"):
     """models/students/depthwise_student.py:187-206 for any callable `model` (windows -> class maps): per image the
     mean over scales of reverse_mapping; returns (N, C, H, W) on the device.  `data` goes through ToPILImage exactly
-    as in the reference (which feeds it the already normalised batch)."""
-    from torchvision import transforms
+    as in the reference (which feeds it the already normalised batch), prepared on the device by prepare_windows: the
+    same windows as the host preparation, without its round trip."""
     mean_std = ([0.485, 0.456, 0.406], [0.229, 0.224, 0.225])
-    to_pil = transforms.ToPILImage()
-    device = data.device
     maps = []
     for x in data:
-        image_data = scale_and_flip_image(to_pil(x.cpu()), mean_std, args['scales'])
-        ori_size, mapping, windows = get_crops_image(image_data, args['scales'], crop_size=args['crop_size'])
-        maps.append(reverse_mapping(mapping, model(windows.to(device)), ori_size, count_mode).mean(dim=0))
+        ori_size, mapping, windows = prepare_windows(x, args['scales'], args['crop_size'], mean_std)
+        maps.append(reverse_mapping(mapping, model(windows), ori_size, count_mode).mean(dim=0))
     return torch.stack(maps)
