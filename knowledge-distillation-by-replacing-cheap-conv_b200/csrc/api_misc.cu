@@ -1,18 +1,9 @@
 // Version / error-string / dispatch-introspection entry points of the C ABI (include/kdcc.h).
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "pw_kernels.cuh"
 #include "sm100_ptx.cuh"
 
 using namespace kdcc;
-
-namespace kdcc {
-bool pdl_enabled() {
-  static const bool on = getenv("KDCC_NO_PDL") == nullptr;
-  return on;
-}
-}  // namespace kdcc
 
 KDCC_API int kdcc_version(void) { return KDCC_VERSION; }
 

@@ -1,22 +1,20 @@
 // C-ABI entry points for the depthwise convolution (declared in include/kdcc.h) and their dispatch:
 //   NCHW bf16                         -> tensor-core kernels (dw_tc.cu, dw_tc_wgrad.cu)
+//   NHWC bf16, 3 x 3, dil 1, pad 1, C / 8 in {2, 4, 8, 16, 32 m} -> streaming 3 x 3 kernels (dw_nhwc3.cu)
 //   NHWC bf16, k in {3, 9}, C % 16 == 0 -> TMA-staged CUDA-core kernels (dw_tma.cu)
 //   NHWC anything else (fp32 parity path, odd kernel sizes) -> direct kernels (dw_direct.cu)
 // There is no CPU or library fallback: unsupported combinations return KDCC_ESHAPE.
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 
 using namespace kdcc;
 
-static bool env_flag(const char *name) {
-  const char *e = getenv(name);
-  return e && atoi(e);
-}
+enum NhwcKernel { NHWC_N3, NHWC_TMA, NHWC_DIRECT };
 
-static bool use_tma(int C, int k, int dil, int dtype) {
-  if (dtype != KDCC_BF16 || env_flag("KDCC_DW_FORCE_DIRECT")) return false;
-  return dw_tma_supported(C, k, dil);
+// the NHWC kernel family that runs for these arguments (a bias gradient always goes to the direct kernel)
+static NhwcKernel nhwc_kernel(int C, int k, int dil, int pad, int dtype) {
+  if (dtype != KDCC_BF16) return NHWC_DIRECT;
+  if (dw_nhwc3_supported(C, k, dil, pad)) return NHWC_N3;
+  return dw_tma_supported(C, k, dil) ? NHWC_TMA : NHWC_DIRECT;
 }
 
 static int check_geometry(int N, int H, int W, int C, int k, int dil, int pad, int layout, int dtype, int *Ho, int *Wo) {
@@ -44,9 +42,9 @@ KDCC_API int kdcc_dw_fwd(const void *x, const float *w, const float *bias, void 
   if (!aligned16(x) || !aligned16(y)) return KDCC_EALIGN;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (layout == KDCC_LAYOUT_NCHW) return dw_tc_conv(x, w, bias, y, N, C, H, W, Ho, Wo, k, dil, pad, 0, st);
-  if (dtype == KDCC_BF16 && dw_nhwc3_supported(C, k, dil, pad) && !env_flag("KDCC_DW_FORCE_DIRECT"))
-    return dw_nhwc3_conv(x, w, bias, y, N, H, W, C, 0, st);
-  if (use_tma(C, k, dil, dtype)) return dw_tma_conv(x, w, bias, y, N, H, W, C, Ho, Wo, k, dil, pad, 0, st);
+  const NhwcKernel kern = nhwc_kernel(C, k, dil, pad, dtype);
+  if (kern == NHWC_N3) return dw_nhwc3_conv(x, w, bias, y, N, H, W, C, 0, st);
+  if (kern == NHWC_TMA) return dw_tma_conv(x, w, bias, y, N, H, W, C, Ho, Wo, k, dil, pad, 0, st);
   if (dtype == KDCC_F32) return dw_direct_fwd<float>(x, w, bias, y, N, H, W, C, Ho, Wo, k, dil, pad, 0, st);
   return dw_direct_fwd<__nv_bfloat16>(x, w, bias, y, N, H, W, C, Ho, Wo, k, dil, pad, 0, st);
 }
@@ -59,13 +57,16 @@ KDCC_API size_t kdcc_dw_bwd_workspace_bytes(int N, int H, int W, int C, int k, i
     const size_t a = dw_tc_wgrad_workspace(N, C, Ho, Wo, k), b = dw_tc_wgrad2_workspace(N, C, k), c = dw_tc_wgrad3_workspace(N, C);
     return a > b ? (a > c ? a : c) : (b > c ? b : c);
   }
+  // bound over every weight-gradient kernel that may run: the direct one (bias gradients) for any shape, the TMA
+  // one's splits for every TMA shape (each streaming 3 x 3 shape is one), the streaming one's CTAs
+  const NhwcKernel kern = nhwc_kernel(C, k, dil, pad, dtype);
   const int vn = dtype == KDCC_F32 ? 4 : 8;
   size_t splits = (size_t)dw_direct_wgrad_splits(N, Ho, C, k, vn);
-  if (dtype == KDCC_BF16 && dw_tma_supported(C, k, dil)) {
+  if (kern != NHWC_DIRECT) {
     const size_t s2 = (size_t)dw_tma_wgrad_splits(N, Ho, Wo, C, k, dil);
     if (s2 > splits) splits = s2;
   }
-  if (dtype == KDCC_BF16 && dw_nhwc3_supported(C, k, dil, pad)) {
+  if (kern == NHWC_N3) {
     const size_t s3 = (size_t)dw_nhwc3_wgrad_ctas(N, H, W, C);
     if (s3 > splits) splits = s3;
   }
@@ -102,9 +103,8 @@ KDCC_API int kdcc_dw_bwd(const void *x, const float *w, const void *dy, void *dx
     }
     return KDCC_OK;
   }
-  const bool tma = use_tma(C, k, dil, dtype);
-  const bool n3 = dtype == KDCC_BF16 && dw_nhwc3_supported(C, k, dil, pad) && !env_flag("KDCC_DW_FORCE_DIRECT");
-  if (n3) {  // streaming 3 x 3 kernels: dX is the conv over dy with mirrored taps (pad' = 1), dW its own kernel
+  const NhwcKernel kern = nhwc_kernel(C, k, dil, pad, dtype);
+  if (kern == NHWC_N3) {  // streaming 3 x 3 kernels: dX is the conv over dy with mirrored taps (pad' = 1), dW its own kernel
     if (dx) {
       rc = dw_nhwc3_conv(dy, w, nullptr, dx, N, H, W, C, 1, st);
       if (rc) return rc;
@@ -114,14 +114,14 @@ KDCC_API int kdcc_dw_bwd(const void *x, const float *w, const void *dy, void *dx
     dx = nullptr;  // bias gradient requested: the direct weight-gradient kernel produces dw and dbias together
   }
   if (dx) {
-    if (tma && padt >= 0) rc = dw_tma_conv(dy, w, nullptr, dx, N, Ho, Wo, C, H, W, k, dil, padt, 1, st);
+    if (kern == NHWC_TMA && padt >= 0) rc = dw_tma_conv(dy, w, nullptr, dx, N, Ho, Wo, C, H, W, k, dil, padt, 1, st);
     else if (dtype == KDCC_F32) rc = dw_direct_fwd<float>(dy, w, nullptr, dx, N, Ho, Wo, C, H, W, k, dil, padt, 1, st);
     else rc = dw_direct_fwd<__nv_bfloat16>(dy, w, nullptr, dx, N, Ho, Wo, C, H, W, k, dil, padt, 1, st);
     if (rc) return rc;
   }
   if (dw || dbias) {
     float *part = static_cast<float *>(workspace);
-    if (tma && !dbias) rc = dw_tma_wgrad(x, dy, dw, part, N, H, W, C, Ho, Wo, k, dil, pad, st);
+    if (kern == NHWC_TMA && !dbias) rc = dw_tma_wgrad(x, dy, dw, part, N, H, W, C, Ho, Wo, k, dil, pad, st);
     else if (dtype == KDCC_F32) rc = dw_direct_wgrad<float>(x, dy, dw, dbias, part, N, H, W, C, Ho, Wo, k, dil, pad, st);
     else rc = dw_direct_wgrad<__nv_bfloat16>(x, dy, dw, dbias, part, N, H, W, C, Ho, Wo, k, dil, pad, st);
     if (rc) return rc;

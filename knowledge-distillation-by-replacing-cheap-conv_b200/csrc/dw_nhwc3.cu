@@ -18,8 +18,6 @@
 //  * weight gradient: same walk, the arriving x row meets the three dy rows around it; 9 x 8 partial sums per
 //    thread over ALL the tiles of a persistent CTA, then a fixed-order shared-memory sum over the CTA's columns and
 //    one partial per CTA (deterministic two-stage reduction, no atomics).
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "sm100_ptx.cuh"
 
@@ -53,7 +51,7 @@ struct N3Params {
   int tiles_h, tiles_w;      // tile = N3_TH rows x N3_WARPS * Jb columns
   int flip;
   int ctas_per_group;        // persistent CTAs per channel group
-  int prefill;               // ring stages filled ahead: stages - lag (the producer refills a stage `lag` arrivals after it was read)
+  int prefill;               // ring stages filled ahead: stages - 1 (the producer refills a stage one arrival after it was read)
   int dbg;                   // KDCC_TC_DEBUG (timing experiments): 1 skip the FMAs, 2 skip the TMA ring (compute on stale smem), 4 skip stores
 };
 
@@ -353,15 +351,9 @@ dw_nhwc3_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
 // host side
 // ------------------------------------------------------------------------------------------------
 bool dw_nhwc3_supported(int C, int k, int dil, int pad) {
-  if (getenv("KDCC_DW_NHWC3_OFF")) return false;
   if (k != 3 || dil != 1 || pad != 1 || C % 8 != 0) return false;
   const int V = C / N3_CH;
   return V % 32 == 0 || V == 2 || V == 4 || V == 8 || V == 16;  // (V == 1 would need a TMA box wider than 256 columns)
-}
-
-static int n3_lag() {  // measurement knob; the default is what bench.py and the tests run
-  const char *e = getenv("KDCC_N3_LAG");
-  return e ? max(1, atoi(e)) : 1;
 }
 
 static void n3_geometry(N3Params &p) {
@@ -392,7 +384,7 @@ int dw_nhwc3_conv(const void *in, const float *w, const float *bias, void *out, 
   if ((long)N * H * W == 0) return KDCC_OK;
   p.dbg = tc_debug_bits();
   CUtensorMap tm;
-  p.prefill = max(1, N3_STAGES - n3_lag());
+  p.prefill = N3_STAGES - 1;
   int rc = n3_map(&tm, in, p, N3_WARPS * p.Jb + 2);
   if (rc) return rc;
   const int smem = N3_STAGES * (((N3_WARPS * p.Jb + 2) * p.Vb * N3_VB + 127) & ~127) + 2 * N3_BAR;
@@ -413,7 +405,7 @@ int dw_nhwc3_wgrad(const void *x, const void *dy, float *dw, float *part, int N,
   N3Params p{};
   p.part = part; p.N = N; p.H = H; p.W = W; p.C = C;
   n3_geometry(p);
-  p.prefill = max(1, N3_WSTAGES - n3_lag());
+  p.prefill = N3_WSTAGES - 1;
   CUtensorMap tm_x, tm_dy;
   int rc = n3_map(&tm_x, x, p, N3_WARPS * p.Jb + 2);
   if (rc) return rc;

@@ -14,7 +14,6 @@
 //    a +128*u*d byte bump of the UMMA descriptor start address, the column slice of an output N-tile a
 //    +32 byte bump.  No im2col, no data movement.  (TMA needs a 16-byte aligned column origin, so the window
 //    starts up to 7 columns left of j0 - pad and the Toeplitz band is shifted right by the same amount.)
-//    KDCC_DW_TC_SINGLE=0 selects the conservative variant that lands one aligned 128-row tile per tap row.
 //  * B_u (16 x 64 bf16, 2 KB) is the Toeplitz band of one tap row; the band positions are identical for
 //    every channel, so the buffers are zeroed once and only the k*16*k band values are rewritten per plane.
 //  * D (128 x 128 fp32) lives in TMEM, double buffered: the epilogue of plane n overlaps the MMAs of n+1.
@@ -22,8 +21,6 @@
 // for the current one (tcgen05.ld -> bf16 -> global).
 // The input-gradient form is the same kernel over dy with mirrored taps (flip) and pad' = d(k-1) - pad.
 // Reference semantics: models/students/transform_blocks/depthwise_separable_conv.py:7-8,12 (+ autograd).
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "dw_tc_common.cuh"
 #include "sm100_ptx.cuh"
@@ -32,17 +29,16 @@ namespace kdcc {
 
 constexpr int TC_TILE = 128;     // output rows and columns per tile (UMMA M = 128)
 constexpr int TC_THREADS = 288;  // warp 0 TMA, warps 1,6,7,8 MMA issuers (N-tiles round-robin), warps 2-5 epilogue
+constexpr int TC_ISSUERS = 4;    // MMA-issuing threads: lane 0 of warps 1, 6, 7, 8
 
 struct DwTcParams {
   int N, C, Hi, Wi, Ho, Wo, k, dil, pad, flip;
   int halo;       // dil * (k - 1)
   int nbox;       // 64-column boxes per A tile
   int a_stages;   // A tiles in flight
-  int single;     // 1: one (128+halo)-row window per item, tap rows are descriptor row shifts; 0: one tile per tap row
-  int rows;       // rows per A tile: 128 (+ halo when single)
+  int rows;       // rows per A tile: 128 + halo, the input window of one item
   int box_bytes;  // ceil8(rows) * 128
   int extra;      // zero columns added on the left so that the TMA column origin is 16-byte aligned
-  int issuers;    // MMA-issuing threads (1, 2 or 4)
   int ksteps;     // ceil((NT + halo) / 16)
   int tiles_h, tiles_w;
   int planes, splits;  // planes per channel (N * tiles), CTAs sharing a channel
@@ -103,19 +99,19 @@ dw_tc_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const DwTcParams p)
   auto t_full = [&](int s) { return bar_base + 8u * (2 + s); };
   auto t_empty = [&](int s) { return bar_base + 8u * (4 + s); };
   auto a_full = [&](int s) { return bar_base + 8u * (6 + s); };
-  auto a_empty = [&](int s) { return bar_base + 8u * (6 + 8 + s); };  // up to 8 A stages
+  auto a_empty = [&](int s) { return bar_base + 8u * (6 + 8 + s); };  // room for 8 A stages (2 in use)
   volatile uint32_t *tmem_slot = reinterpret_cast<volatile uint32_t *>(smem_gen + (bar_base - smem_base) + 8 * 22);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
     for (int s = 0; s < 2; ++s) {
       ptx::mbar_init(b_full(s), 128);
-      ptx::mbar_init(t_full(s), p.issuers);   // one commit per issuing thread
+      ptx::mbar_init(t_full(s), TC_ISSUERS);   // one commit per issuing thread
       ptx::mbar_init(t_empty(s), 4);
     }
     for (int s = 0; s < AS; ++s) {
       ptx::mbar_init(a_full(s), 1);
-      ptx::mbar_init(a_empty(s), p.issuers);
+      ptx::mbar_init(a_empty(s), TC_ISSUERS);
     }
     ptx::fence_barrier_init();
     ptx::prefetch_tensormap(&tm_in);
@@ -135,26 +131,22 @@ dw_tc_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const DwTcParams p)
   };
 
   if (warp == 0 && lane == 0) {
-    // ===== TMA producer: the input window of an item, once (single) or once per tap row =====
+    // ===== TMA producer: the input window of an item, once =====
     int as = 0; uint32_t aph = 0;
-    const int tiles = p.single ? 1 : p.k;
     for (PlaneWalk w(p.pairs, p.planes, p.splits, p.C); w.valid(); w.next()) {
       const int c = w.channel();
       int n, i0, j0;
       decode(w.pl, n, i0, j0);
-      for (int u = 0; u < tiles; ++u) {
-        ptx::mbar_wait(a_empty(as), aph ^ 1);
-        ptx::mbar_arrive_expect_tx(a_full(as), (uint32_t)(p.nbox * p.rows * 128));
-        for (int b = 0; b < p.nbox; ++b)
-          ptx::tma_load_4d(smem_base + as * a_stage_bytes + b * p.box_bytes, &tm_in, a_full(as),
-                           j0 - p.pad - p.extra + 64 * b, i0 - p.pad + u * p.dil, c, n);
-        if (++as == AS) { as = 0; aph ^= 1; }
-      }
+      ptx::mbar_wait(a_empty(as), aph ^ 1);
+      ptx::mbar_arrive_expect_tx(a_full(as), (uint32_t)(p.nbox * p.rows * 128));
+      for (int b = 0; b < p.nbox; ++b)
+        ptx::tma_load_4d(smem_base + as * a_stage_bytes + b * p.box_bytes, &tm_in, a_full(as),
+                         j0 - p.pad - p.extra + 64 * b, i0 - p.pad, c, n);
+      if (++as == AS) { as = 0; aph ^= 1; }
     }
-  } else if ((warp == 1 || (warp >= 6 && warp - 5 < p.issuers)) && lane == 0) {
-    // ===== MMA issuers: N-tile t belongs to issuer t % issuers (each tile has its own TMEM columns) =====
+  } else if ((warp == 1 || warp >= 6) && lane == 0) {
+    // ===== MMA issuers: N-tile t belongs to issuer t % TC_ISSUERS (each tile has its own TMEM columns) =====
     const int t_first = warp == 1 ? 0 : warp - 5;
-    const int t_step = p.issuers;
     // instruction descriptor: fp32 accumulate, bf16 x bf16, both K-major, N = NT, M = 128
     constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(TC_TILE >> 4) << 24);
     constexpr int T = TC_TILE / NT;
@@ -184,28 +176,26 @@ dw_tc_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const DwTcParams p)
       }
       const uint32_t b0 = b_base + (unit & 1) * b_stage_bytes;
       const uint32_t d0 = tmem_base + (uint32_t)(s * TC_TILE);
+      ptx::mbar_wait(a_full(as), aph);
+      ptx::tcgen05_fence_after();
 #pragma unroll 1
       for (int u = 0; u < p.k; ++u) {
-        if (!p.single || u == 0) ptx::mbar_wait(a_full(as), aph);
-        ptx::tcgen05_fence_after();
-        // single window: tap row u starts u*dil rows (128 B each) further down the same tile
-        const uint32_t a0 = smem_base + as * a_stage_bytes + (p.single ? (uint32_t)(u * p.dil) * 128u : 0u);
+        // tap row u starts u*dil rows (128 B each) further down the window
+        const uint32_t a0 = smem_base + as * a_stage_bytes + (uint32_t)(u * p.dil) * 128u;
         const uint32_t a_lo = ((a0 & 0x3FFFF) >> 4) | (1u << 16);
         const uint32_t b_lo = (((b0 + (uint32_t)u * BU_BYTES) & 0x3FFFF) >> 4) | b_lbo;
         const uint32_t acc0 = u ? 1u : 0u;
 #pragma unroll
         for (int t = 0; t < T; ++t) {
-          if (t % t_step != t_first || KDCC_DBG(p, 2)) continue;
+          if (t % TC_ISSUERS != t_first || KDCC_DBG(p, 2)) continue;
 #pragma unroll
           for (int kk = 0; kk < KS; ++kk)
             tc_mma(d0 + (uint32_t)(t * NT), a_lo + a_off[t][kk], a_hi, b_lo + (uint32_t)(kk * 2 * NT), b_hi, idesc,
                    kk ? 1u : acc0);
         }
-        if (!p.single || u == p.k - 1) {
-          ptx::umma_commit(a_empty(as));  // tile free once these MMAs have read it
-          if (++as == AS) { as = 0; aph ^= 1; }
-        }
       }
+      ptx::umma_commit(a_empty(as));  // window free once these MMAs have read it
+      if (++as == AS) { as = 0; aph ^= 1; }
       ptx::umma_commit(t_full(s));
     }
   } else if (warp >= 2 && warp <= 5) {
@@ -311,10 +301,10 @@ static int tc_conv_launch(const void *in, const DwTcParams &p0, cudaStream_t st)
   DwTcParams p = p0;
   p.ksteps = KS;
   p.nbox = ceil_div((TC_TILE - NT) + KS * 16, 64);  // the last N-tile's last reduction slice ends here
-  p.rows = TC_TILE + (p.single ? p.halo : 0);
+  p.rows = TC_TILE + p.halo;
   p.box_bytes = (p.rows + 7) / 8 * 8 * 128;
   const int b_bytes = 2 * p.k * KS * 2 * NT * 16;
-  p.a_stages = min(p.single ? 2 : 8, (int)((226 * 1024 - b_bytes - 2048) / (p.nbox * p.box_bytes)));
+  p.a_stages = min(2, (int)((226 * 1024 - b_bytes - 2048) / (p.nbox * p.box_bytes)));
   if (p.a_stages < 2) return KDCC_ESHAPE;
   CUtensorMap tm;
   const uint64_t dims[4] = {(uint64_t)p.Wi, (uint64_t)p.Hi, (uint64_t)p.C, (uint64_t)p.N};
@@ -357,15 +347,7 @@ int dw_tc_conv(const void *in, const float *w, const float *bias, void *out, int
   if (p.planes == 0 || C == 0) return KDCC_OK;
   p.dbg = tc_debug_bits();
   p.extra = tc_extra(pad);
-  const char *is = getenv("KDCC_DW_TC_ISSUERS");
-  p.issuers = is ? max(1, min(4, atoi(is))) : 4;
-  if (p.issuers == 3) p.issuers = 2;
-  const char *sg = getenv("KDCC_DW_TC_SINGLE");
-  p.single = sg ? atoi(sg) : 1;
-  if (TC_TILE + p.halo > 256) p.single = 0;  // TMA box rows
-  const char *e = getenv("KDCC_DW_TC_NT");
-  const int nt = e ? atoi(e) : tc_nt(p.halo + p.extra);
-  if (nt == 32 && p.halo + p.extra + 32 <= 80) return tc_conv_dispatch_ks<32>(in, p, st);
+  if (tc_nt(p.halo + p.extra) == 32) return tc_conv_dispatch_ks<32>(in, p, st);
   return tc_conv_dispatch_ks<16>(in, p, st);
 }
 

@@ -26,8 +26,6 @@
 // windows are 32 phase-columns wide, so a half costs exactly what a 128-column plane costs (90 MMAs) instead of the
 // 180 of the tiled kernel (dw_tc.cu).  Split points are multiples of 5 (phases line up) and of 8 (16-byte store rows).
 // Reference semantics: models/students/transform_blocks/depthwise_separable_conv.py:7-8,12 (+ autograd).
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "dw_tc_common.cuh"
 #include "sm100_ptx.cuh"
@@ -342,12 +340,10 @@ dw_tc_conv2_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_const
 // ------------------------------------------------------------------------------------------------
 // planes of 129 .. 256 columns as two column halves: derived for the 9 x 9, dilation 5, pad 20 geometry (split at column 120)
 static bool conv2_wide(int Hi, int Wi, int Ho, int Wo, int k, int dil, int pad) {
-  return Hi == Ho && Wi == Wo && Hi <= 128 && Wi > 128 && Wi <= 256 && Wi % 8 == 0 && k == 9 && dil == 5 && pad == 20 &&
-         !getenv("KDCC_DW_CONV2_NO_WIDE");
+  return Hi == Ho && Wi == Wo && Hi <= 128 && Wi > 128 && Wi <= 256 && Wi % 8 == 0 && k == 9 && dil == 5 && pad == 20;
 }
 
 bool dw_tc_conv2_supported(int Hi, int Wi, int Ho, int Wo, int k, int dil, int pad) {
-  if (getenv("KDCC_DW_CONV_V1")) return false;
   if (conv2_wide(Hi, Wi, Ho, Wo, k, dil, pad)) return true;
   const int halo = dil * (k - 1);
   if (Hi != Ho || Wi != Wo || Hi > 128 || Wi > 128 || Wi % 8 != 0) return false;

@@ -12,7 +12,6 @@
 // the landed dy tile ONCE per plane into tensor memory (lane = dy column, 64 columns of bf16 pairs) and
 // the MMAs take A from TMEM: the shared-memory operand feed -- the limiter of these small MMAs -- then
 // only carries B.
-// (KDCC_DW_TC_SINGLE=0: conservative variant, one aligned 128-row x tile per tap row.)
 // Only k of the 128+halo columns of each P_u row are needed, so the FFMA-bound CUDA-core formulation
 // (dw_tma.cu: ~14 TFMA/s) is replaced by ~5 % efficient but 50x faster tensor-core work.
 // The epilogue warps pull P_u out of TMEM 32 columns at a time, pick the k diagonal entries of their row
@@ -20,8 +19,6 @@
 // registers across all planes of the channel; a warp-shuffle + fixed-order cross-warp sum finishes the
 // channel.  Deterministic: no atomics, splits (if any) are reduced by dw_wgrad_reduce_kernel.
 // Reference semantics: autograd of models/students/transform_blocks/depthwise_separable_conv.py:12.
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "dw_tc_common.cuh"
 #include "sm100_ptx.cuh"
@@ -35,7 +32,7 @@ constexpr int WG_SCR_PITCH = 36;  // floats per scratch row: 16-byte aligned row
 struct DwTcWgradParams {
   int N, C, H, W, Ho, Wo, k, dil, pad;
   int halo, nbox, x_stages;         // 64-column boxes per x tile, x tiles in flight
-  int single, rows, box_bytes;      // single: one (128+halo)-row window per plane; rows per box; bytes per box
+  int rows, box_bytes;              // rows per box: the (128+halo)-row window of one plane; bytes per box
   int extra;                        // zero columns on the left so that the TMA column origin is 16-byte aligned
   int nq;                           // P_u columns: (128 + halo) rounded up to 16
   int tiles_h, tiles_w, planes;     // planes = N * tiles_h * tiles_w (per channel)
@@ -115,7 +112,7 @@ dw_tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
   auto t_empty = [&](int s) { return bar_base + 8u * (6 + s); };
   auto a_full = [&](int s) { return bar_base + 8u * (8 + s); };   // dy^T of a plane is in TMEM
   auto x_full = [&](int s) { return bar_base + 8u * (10 + s); };
-  auto x_empty = [&](int s) { return bar_base + 8u * (14 + s); };  // up to 4 x stages
+  auto x_empty = [&](int s) { return bar_base + 8u * (14 + s); };  // room for 4 x stages (2 in use)
   volatile uint32_t *tmem_slot = reinterpret_cast<volatile uint32_t *>(smem_gen + bar_off + 160);
   float *red = reinterpret_cast<float *>(smem_gen + bar_off + 192);  // [8 warps][K*K]
 
@@ -151,7 +148,7 @@ dw_tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
   };
 
   if (warp == 0 && lane == 0) {
-    // ===== TMA producer: dy tile once per plane, the x window once per plane (or one tile per tap row) =====
+    // ===== TMA producer: dy tile and x window once per plane =====
     int it = 0;
     int xs = 0; uint32_t xph = 0;
     for (PlaneWalk w(p.pairs, p.planes, p.splits, p.C); w.valid(); w.next(), ++it) {
@@ -164,14 +161,12 @@ dw_tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
       ptx::mbar_arrive_expect_tx(dy_full(0), 2 * WG_BOX);
       for (int b = 0; b < 2; ++b)
         ptx::tma_load_4d(smem_base + dy_off + b * WG_BOX, &tm_dy, dy_full(0), j0 + 64 * b, i0, c, n);
-      for (int u = 0; u < (p.single ? 1 : K); ++u) {
-        ptx::mbar_wait(x_empty(xs), xph ^ 1);
-        ptx::mbar_arrive_expect_tx(x_full(xs), (uint32_t)(p.nbox * p.rows * 128));
-        for (int b = 0; b < p.nbox; ++b)
-          ptx::tma_load_4d(smem_base + xs * x_bytes + b * p.box_bytes, &tm_x, x_full(xs),
-                           j0 - p.pad - p.extra + 64 * b, i0 - p.pad + u * p.dil, c, n);
-        if (++xs == XS) { xs = 0; xph ^= 1; }
-      }
+      ptx::mbar_wait(x_empty(xs), xph ^ 1);
+      ptx::mbar_arrive_expect_tx(x_full(xs), (uint32_t)(p.nbox * p.rows * 128));
+      for (int b = 0; b < p.nbox; ++b)
+        ptx::tma_load_4d(smem_base + xs * x_bytes + b * p.box_bytes, &tm_x, x_full(xs),
+                         j0 - p.pad - p.extra + 64 * b, i0 - p.pad, c, n);
+      if (++xs == XS) { xs = 0; xph ^= 1; }
     }
   } else if (warp == 1 && lane == 0) {
     // ===== MMA issuer: P_u (128 dy columns x nq window columns) = dy^T [TMEM] * x_u [smem, MN-major] =====
@@ -187,12 +182,12 @@ dw_tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
       const uint32_t a_tmem = tmem_base + (s ? WG_TMEM_A1 : WG_TMEM_A0);
       for (int u = 0; u < K; ++u, ++tit) {
         const int tb = tit & 1;
-        if (!p.single || u == 0) ptx::mbar_wait(x_full(xs), xph);
+        if (u == 0) ptx::mbar_wait(x_full(xs), xph);  // inside the loop: hoisted, it costs the K = 9 instance a spill
         ptx::mbar_wait(t_empty(tb), ((tit >> 1) & 1) ^ 1);
         ptx::tcgen05_fence_after();
         const uint32_t d_tmem = tmem_base + (tb ? WG_TMEM_D1 : 0u);
-        // single window: tap row u starts u*dil rows (128 B each) further down the same tile
-        const uint32_t xa = smem_base + xs * x_bytes + (p.single ? (uint32_t)(u * p.dil) * 128u : 0u);
+        // tap row u starts u*dil rows (128 B each) further down the window
+        const uint32_t xa = smem_base + xs * x_bytes + (uint32_t)(u * p.dil) * 128u;
         const uint32_t b_lo = ((xa & 0x3FFFF) >> 4) | ((uint32_t)(p.box_bytes >> 4) << 16);
         if (!KDCC_DBG(p, 2)) {
 #pragma unroll
@@ -200,8 +195,8 @@ dw_tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
             wg_mma_ts(d_tmem, a_tmem + ks * 8, b_lo + ks * 128, b_hi, idesc, ks ? 1u : 0u);
         }
         ptx::umma_commit(t_full(tb));
-        if (!p.single || u == K - 1) {
-          ptx::umma_commit(x_empty(xs));
+        if (u == K - 1) {
+          ptx::umma_commit(x_empty(xs));  // window free once the last tap row's MMAs have read it
           if (++xs == XS) { xs = 0; xph ^= 1; }
         }
       }
@@ -342,7 +337,7 @@ static int wgrad_launch(const void *x, const void *dy, float *dw, float *part, c
   }
   p.out = p.splits == 1 ? dw : part;
   const int fixed = 2 * WG_BOX + 8 * 32 * WG_SCR_PITCH * 4 + 192 + 8 * K * K * 4 + 64 + 1024;  // dy, scratch, barriers, red, slack
-  p.x_stages = min(p.single ? 2 : 4, (220 * 1024 - fixed) / (p.nbox * p.box_bytes));
+  p.x_stages = min(2, (220 * 1024 - fixed) / (p.nbox * p.box_bytes));
   if (p.x_stages < 2) return KDCC_ESHAPE;
   const int smem = p.x_stages * p.nbox * p.box_bytes + fixed;
   static int attr_cache[16] = {0};
@@ -365,10 +360,7 @@ int dw_tc_wgrad(const void *x, const void *dy, float *dw, float *part, int N, in
   p.extra = (8 - pad % 8) % 8;
   p.nq = (WG_TILE + p.halo + p.extra + 15) / 16 * 16;
   p.nbox = ceil_div(p.nq, 64);
-  const char *sg = getenv("KDCC_DW_TC_SINGLE");
-  p.single = sg ? atoi(sg) : 1;
-  if (WG_TILE + p.halo > 256) p.single = 0;
-  p.rows = WG_TILE + (p.single ? p.halo : 0);
+  p.rows = WG_TILE + p.halo;
   p.box_bytes = (p.rows + 7) / 8 * 8 * 128;
   p.tiles_h = ceil_div(Ho, WG_TILE);
   p.tiles_w = ceil_div(Wo, WG_TILE);

@@ -17,8 +17,6 @@
 // landing tile (32 KB), scratch (18 KB).  TMEM: dy^T of 2 stages x 2 planes (256 columns) + 2 x P_u (256 columns).
 // Deterministic: fixed-order sums, no atomics; splits are reduced by dw_tc_wgrad_reduce (dw_tc_wgrad.cu).
 // Reference semantics: autograd of models/students/transform_blocks/depthwise_separable_conv.py:12.
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "dw_tc_common.cuh"
 #include "sm100_ptx.cuh"
@@ -260,7 +258,6 @@ dw_tc_wgrad2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
 // ------------------------------------------------------------------------------------------------
 bool dw_tc_wgrad2_supported(int H, int W, int Ho, int Wo, int k, int dil, int pad) {
   const int halo = dil * (k - 1);
-  if (getenv("KDCC_DW_WGRAD_V1")) return false;
   return H == Ho && W == Wo && H <= 128 && W <= 128 && W % 8 == 0 && k % 2 == 1 && k <= 9 && pad <= W2_GAP &&
          halo - pad >= 0 && halo - pad <= W2_GAP;
 }

@@ -43,8 +43,6 @@
 // the MMAs down, but beside them a warp gets one x32 load per ~240 clk (tools/tc_probe2 "ts 128 32 3 1 8": 134 B/clk/SM for
 // eight warps, 239 idle): the converters' 320 KB per plane are latency-, not bandwidth-bound.
 // Reference semantics: autograd of models/students/transform_blocks/depthwise_separable_conv.py:12.
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "dw_tc_common.cuh"
 #include "sm100_ptx.cuh"
@@ -435,7 +433,6 @@ dw_tc_wgrad3_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
 // host side
 // ------------------------------------------------------------------------------------------------
 bool dw_tc_wgrad3_supported(int H, int W, int Ho, int Wo, int k, int dil, int pad) {
-  if (getenv("KDCC_DW_WGRAD_V2") || getenv("KDCC_DW_WGRAD_V1")) return false;
   return H == Ho && W == Wo && H <= 128 && W <= 128 && W % 8 == 0 && k == W3_K && dil == W3_D && pad == W3_PAD;
 }
 

@@ -19,8 +19,6 @@
 //  * Weight gradient: same staging for x, dy read straight from its bf16 landing tile; each thread owns
 //    (channel pair, tap row u) and keeps K x 2 partial sums in registers across ALL the tiles of its
 //    CTA; cross-thread / cross-CTA reduction is a fixed-order two-stage sum (deterministic, no atomics).
-#include <stdlib.h>
-
 #include "dw_kernels.cuh"
 #include "sm100_ptx.cuh"
 
@@ -67,15 +65,12 @@ using Cfg9 = DwCfg<9, 26, 26, 13, 16, 3, 1>;  // Cityscapes cfgs: k=9, dil=5, pa
 using Cfg3 = DwCfg<3, 16, 32, 8, 16, 4, 2>;   // CIFAR / north-star 3x3
 
 struct DwTmaParams {
-  int N, Hi, Wi, Ho, Wo, C, dil, pad, flip;
+  int N, C, dil, pad, flip;
   int tiles_h, tiles_w, ncb;
   long total;  // conv: all tiles; wgrad: spatial tiles (without the channel-block factor)
   int splits;  // wgrad: CTAs per channel block
   const float *w, *bias;
-  const __nv_bfloat16 *in;
-  __nv_bfloat16 *out;
   float *part;
-  int mode;  // debug: bit0 = plain-load staging instead of TMA, bit1 = plain stores instead of TMA store
 };
 
 struct TileCoord {
@@ -110,21 +105,6 @@ __device__ __forceinline__ void widen_tile(const uint8_t *land, float *f32, int 
   }
 }
 
-// debug/insurance staging without TMA: gathers the strided sub-image with plain 16-byte loads
-template <int ROWS, int COLS, int CB, int NT>
-__device__ __forceinline__ void manual_stage(uint8_t *land, const __nv_bfloat16 *src, int n, int H, int W, int C,
-                                             int r0, int c0, int dil, int cb, int tid) {
-  constexpr int CHUNKS = ROWS * COLS * (CB / 8);
-  for (int i = tid; i < CHUNKS; i += NT) {
-    const int px = i / (CB / 8), ch = i % (CB / 8);
-    const int gi = r0 + (px / COLS) * dil, gj = c0 + (px % COLS) * dil;
-    uint4 v = make_uint4(0, 0, 0, 0);
-    if (gi >= 0 && gi < H && gj >= 0 && gj < W)
-      v = *reinterpret_cast<const uint4 *>(src + (((long)n * H + gi) * W + gj) * C + cb * CB + ch * 8);
-    *reinterpret_cast<uint4 *>(land + (size_t)i * 16) = v;
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // forward / input-gradient kernel
 // ------------------------------------------------------------------------------------------------
@@ -140,7 +120,6 @@ dw_tma_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_const
   float *wsm = reinterpret_cast<float *>(smem + Cfg::CONV_OFF_W);
   const uint32_t bar0 = ptx::smem_u32(smem + Cfg::CONV_OFF_BAR);
   const int tid = threadIdx.x;
-  const bool manual_load = p.mode & 1, manual_store = p.mode & 2;
 
   if (tid == 0) {
     ptx::mbar_init(bar0, 1);
@@ -157,7 +136,7 @@ dw_tma_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_const
     ptx::mbar_arrive_expect_tx(bar, Cfg::LAND_BYTES);
     ptx::tma_load_4d(ptx::smem_u32(land[stage]), &tm_in, bar, tc.cb * CB, tc.j0 - p.pad, tc.i0 - p.pad, tc.n);
   };
-  if (tid == 0 && !manual_load) {
+  if (tid == 0) {
     for (int s = 0; s < 2; ++s) {
       const long tile = (long)blockIdx.x + (long)s * gridDim.x;
       if (tile < p.total) issue_load(tile, s);
@@ -184,13 +163,7 @@ dw_tma_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_const
       else v = p.bias ? __ldg(p.bias + tc.cb * CB + c) : 0.f;
       wsm[i] = v;
     }
-    if (manual_load) {
-      manual_stage<Cfg::IH, Cfg::IW, CB, NT>(land[st], p.in, tc.n, p.Hi, p.Wi, p.C, tc.i0 - p.pad, tc.j0 - p.pad,
-                                             p.dil, tc.cb, tid);
-      __syncthreads();
-    } else {
-      ptx::mbar_wait(bar0 + 8 * st, phase);
-    }
+    ptx::mbar_wait(bar0 + 8 * st, phase);
     widen_tile<Cfg, NT>(land[st], f32, tid);
     if (tid == 0) ptx::tma_store_wait_read();  // the previous tile's store has drained the out tile
     __syncthreads();
@@ -226,27 +199,14 @@ dw_tma_conv_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_const
 #pragma unroll
       for (int t = 0; t < T; ++t) orow_ptr[t * CP] = pack_bf16x2(acc[t][0], acc[t][1]);
     }
-    if (!manual_store) ptx::fence_proxy_async_smem();
+    ptx::fence_proxy_async_smem();
     __syncthreads();
 
-    if (manual_store) {
-      constexpr int CHUNKS = Cfg::TH * Cfg::TW * (CB / 8);
-      for (int i = tid; i < CHUNKS; i += NT) {
-        const int px = i / (CB / 8), ch = i % (CB / 8);
-        const int gi = tc.i0 + (px / Cfg::TW) * p.dil, gj = tc.j0 + (px % Cfg::TW) * p.dil;
-        if (gi < p.Ho && gj < p.Wo)
-          *reinterpret_cast<uint4 *>(p.out + (((long)tc.n * p.Ho + gi) * p.Wo + gj) * p.C + tc.cb * CB + ch * 8) =
-              *reinterpret_cast<const uint4 *>(reinterpret_cast<const uint8_t *>(outs) + (size_t)i * 16);
-      }
-      __syncthreads();
-    }
     if (tid == 0) {
-      if (!manual_store) {
-        ptx::tma_store_4d(&tm_out, ptx::smem_u32(outs), tc.cb * CB, tc.j0, tc.i0, tc.n);
-        ptx::tma_store_commit();
-      }
+      ptx::tma_store_4d(&tm_out, ptx::smem_u32(outs), tc.cb * CB, tc.j0, tc.i0, tc.n);
+      ptx::tma_store_commit();
       const long next = tile + 2L * gridDim.x;
-      if (!manual_load && next < p.total) issue_load(next, st);
+      if (next < p.total) issue_load(next, st);
     }
   }
   if (tid == 0) ptx::tma_store_wait_all();
@@ -267,7 +227,6 @@ dw_tma_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
   float *f32 = reinterpret_cast<float *>(smem + Cfg::WG_OFF_F32);
   const uint32_t bar0 = ptx::smem_u32(smem + Cfg::WG_OFF_BAR);
   const int tid = threadIdx.x;
-  const bool manual_load = p.mode & 1;
   const int cb = blockIdx.x % p.ncb;
   const int split = blockIdx.x / p.ncb;
 
@@ -287,7 +246,7 @@ dw_tma_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
     ptx::tma_load_4d(ptx::smem_u32(landx[stage]), &tm_x, bar, cb * CB, tc.j0 - p.pad, tc.i0 - p.pad, tc.n);
     ptx::tma_load_4d(ptx::smem_u32(landg[stage]), &tm_dy, bar, cb * CB, tc.j0, tc.i0, tc.n);
   };
-  if (tid == 0 && !manual_load) {
+  if (tid == 0) {
     for (int s = 0; s < 2; ++s) {
       const long tile = (long)split + (long)s * p.splits;
       if (tile < p.total) issue_load(tile, s);
@@ -312,15 +271,7 @@ dw_tma_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
   for (long tile = split; tile < p.total; tile += p.splits, ++it) {
     const int st = it & 1;
     const uint32_t phase = (it >> 1) & 1;
-    if (manual_load) {
-      const TileCoord tc = decode_tile<Cfg>(p, tile, false);
-      manual_stage<Cfg::IH, Cfg::IW, CB, NT>(landx[st], p.in, tc.n, p.Hi, p.Wi, p.C, tc.i0 - p.pad, tc.j0 - p.pad,
-                                             p.dil, cb, tid);
-      manual_stage<Cfg::TH, Cfg::TW, CB, NT>(landg[st], p.out, tc.n, p.Ho, p.Wo, p.C, tc.i0, tc.j0, p.dil, cb, tid);
-      __syncthreads();
-    } else {
-      ptx::mbar_wait(bar0 + 8 * st, phase);
-    }
+    ptx::mbar_wait(bar0 + 8 * st, phase);
     widen_tile<Cfg, NT>(landx[st], f32, tid);
     __syncthreads();
 
@@ -352,7 +303,7 @@ dw_tma_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
       }
     }
     __syncthreads();
-    if (tid == 0 && !manual_load) {
+    if (tid == 0) {
       const long next = tile + 2L * p.splits;
       if (next < p.total) issue_load(next, st);
     }
@@ -378,11 +329,6 @@ dw_tma_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static int debug_mode() {
-  const char *e = getenv("KDCC_DW_MODE");
-  return e ? atoi(e) : 0;
-}
-
 // 4-D map over an NHWC bf16 tensor; box = (CB, cols*dil, rows*dil, 1) traversed with stride dil
 static int nhwc_map(CUtensorMap *m, const void *base, int N, int H, int W, int C, int cb, int rows, int cols, int dil) {
   const uint64_t dims[4] = {(uint64_t)C, (uint64_t)W, (uint64_t)H, (uint64_t)N};
@@ -411,22 +357,19 @@ const char *dw_tma_name(int k, int dil, int which) {
 }
 
 template <class Cfg>
-static void fill_geometry(DwTmaParams &p, int N, int Hi, int Wi, int C, int Ho, int Wo, int dil, int pad) {
-  p.N = N; p.Hi = Hi; p.Wi = Wi; p.Ho = Ho; p.Wo = Wo; p.C = C; p.dil = dil; p.pad = pad;
+static void fill_geometry(DwTmaParams &p, int N, int C, int Ho, int Wo, int dil, int pad) {
+  p.N = N; p.C = C; p.dil = dil; p.pad = pad;
   p.tiles_h = ceil_div(ceil_div(Ho, dil), Cfg::TH);
   p.tiles_w = ceil_div(ceil_div(Wo, dil), Cfg::TW);
   p.ncb = C / Cfg::CB;
-  p.mode = debug_mode();
 }
 
 template <class Cfg>
 static int conv_launch(const void *in, const float *w, const float *bias, void *out, int N, int Hi, int Wi, int C,
                        int Ho, int Wo, int dil, int pad, int flip, cudaStream_t st) {
   DwTmaParams p{};
-  fill_geometry<Cfg>(p, N, Hi, Wi, C, Ho, Wo, dil, pad);
+  fill_geometry<Cfg>(p, N, C, Ho, Wo, dil, pad);
   p.flip = flip; p.w = w; p.bias = bias;
-  p.in = static_cast<const __nv_bfloat16 *>(in);
-  p.out = static_cast<__nv_bfloat16 *>(out);
   p.total = (long)N * dil * dil * p.tiles_h * p.tiles_w * p.ncb;
   if (p.total == 0) return KDCC_OK;
   CUtensorMap tm_in, tm_out;
@@ -464,9 +407,7 @@ template <class Cfg>
 static int wgrad_launch(const void *x, const void *dy, float *dw, float *part, int N, int H, int W, int C, int Ho,
                         int Wo, int dil, int pad, cudaStream_t st) {
   DwTmaParams p{};
-  fill_geometry<Cfg>(p, N, H, W, C, Ho, Wo, dil, pad);
-  p.in = static_cast<const __nv_bfloat16 *>(x);
-  p.out = const_cast<__nv_bfloat16 *>(static_cast<const __nv_bfloat16 *>(dy));
+  fill_geometry<Cfg>(p, N, C, Ho, Wo, dil, pad);
   p.part = part;
   p.total = (long)N * dil * dil * p.tiles_h * p.tiles_w;
   p.splits = wgrad_splits<Cfg>(N, Ho, Wo, C, dil);

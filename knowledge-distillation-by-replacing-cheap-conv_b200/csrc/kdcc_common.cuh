@@ -22,13 +22,11 @@ static inline int launch_status() {
 // Kernels launched through launch_pdl may become resident while their predecessor in the stream is still running:
 // their prologue (shared-memory fills, barrier init, TMEM allocation, descriptor prefetch) overlaps its tail.  Every
 // such kernel calls pdl_prologue_done() before its first global-memory access: it lets ITS dependents start early and
-// then waits until the predecessor grid has completed and flushed.  KDCC_NO_PDL=1 restores plain stream order.
+// then waits until the predecessor grid has completed and flushed.
 __device__ __forceinline__ void pdl_prologue_done() {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   asm volatile("griddepcontrol.wait;" ::: "memory");
 }
-
-bool pdl_enabled();  // api_misc.cu
 
 template <typename... KArgs, typename... Args>
 static inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
@@ -41,7 +39,7 @@ static inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -2,16 +2,12 @@
 // bf16 -> tcgen05/TMEM GEMM (pw_gemm_sm100.cu); KDCC_F32_TF32X3 -> fp32 as three tf32 tcgen05 products
 // (pw_gemm_tf32x3.cu); fp32 (parity path) and channel counts the tensor-core kernels do not take -> CUDA-core GEMM
 // (pw_gemm_simt.cu).  No CPU / library fallback.
-#include <stdlib.h>
-
 #include "pw_kernels.cuh"
 
 using namespace kdcc;
 
 static bool use_sm100(long M, int K, int Nc, int batch, int layout, int dtype) {
   if (dtype != KDCC_BF16) return false;
-  const char *e = getenv("KDCC_PW_FORCE_SIMT");
-  if (e && atoi(e) && layout == KDCC_LAYOUT_NHWC) return false;
   return pw_sm100_supported(M, K, Nc, batch, layout);
 }
 

@@ -18,8 +18,6 @@
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer (one lane),
 // warps 2..5 = epilogue (one TMEM lane quadrant each).  Persistent CTAs walk work items round-robin;
 // the accumulator is double-buffered in TMEM so the epilogue of item n overlaps the MMAs of item n+1.
-#include <stdlib.h>
-
 #include "kdcc_common.cuh"
 #include "pw_kernels.cuh"
 #include "sm100_ptx.cuh"
@@ -397,7 +395,7 @@ static int gemm_launch(const void *a, const void *b, const GemmParams &p0, cudaS
   // bf16 raw output only: TMA-store epilogue over out[batch][I][J]
   CUtensorMap tm_out = tm_a;
   p.tma_out = 0;
-  if (p.out_raw && !p.out_act && !p.out_f32 && !getenv("KDCC_PW_DIRECT_STORE")) {
+  if (p.out_raw && !p.out_act && !p.out_f32) {
     const int ob = p.r_spans_batch ? 1 : p.batch;
     const uint64_t dims[3] = {(uint64_t)p.J, (uint64_t)p.I, (uint64_t)ob};
     const uint64_t strides[2] = {(uint64_t)p.J * 2, (uint64_t)(ob > 1 ? p.out_batch_stride : (long)p.I * p.J) * 2};
@@ -426,7 +424,7 @@ static int gemm_launch(const void *a, const void *b, const GemmParams &p0, cudaS
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 2;
   cudaLaunchKernelEx(&cfg, pw_gemm_sm100_kernel<BJ, A_MN, B_MN, PAIR>, tm_a, tm_b, tm_out, p);
   return launch_status();
 }
@@ -434,8 +432,8 @@ static int gemm_launch(const void *a, const void *b, const GemmParams &p0, cudaS
 template <bool A_MN, bool B_MN>
 static int gemm_dispatch_bj(const void *a, const void *b, const GemmParams &p, cudaStream_t st) {
   if (p.J >= 256 && p.J % 256 == 0) {
-    // CTA pairs need an even number of 128-row tiles; KDCC_PW_1CTA=1 keeps the single-CTA kernel (A/B measurements)
-    if (ceil_div(p.I, GEMM_BI) % 2 == 0 && !getenv("KDCC_PW_1CTA")) return gemm_launch<256, A_MN, B_MN, true>(a, b, p, st);
+    // CTA pairs need an even number of 128-row tiles
+    if (ceil_div(p.I, GEMM_BI) % 2 == 0) return gemm_launch<256, A_MN, B_MN, true>(a, b, p, st);
     return gemm_launch<256, A_MN, B_MN, false>(a, b, p, st);
   }
   if (p.J > 64) return gemm_launch<128, A_MN, B_MN, false>(a, b, p, st);

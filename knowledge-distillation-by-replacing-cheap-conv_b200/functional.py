@@ -15,8 +15,6 @@ Reference call sites replaced (reference file:line):
   canny_edges         models/gscnn/gscnn.py:284-288 (uint8 cast + cv2.Canny per image, without the host round trip)
   tta_windows         utils/tta_process.py:52-117 (PIL rescale, mirror, normalise and window crops, without the host round trip)
 """
-import os
-
 import torch
 
 from . import _abi
@@ -215,7 +213,7 @@ class _DepthwiseConv(torch.autograd.Function):
         if bias is None and _supported(0, N, H, W, C, C, k, dil, pad, _abi.NCHW, code):
             if _is_plain_nchw(x):
                 layout = _abi.NCHW
-            elif k > 3 and _is_channels_last(x) and _convertible(x) and not os.environ.get("KDCC_DW_KEEP_NHWC"):
+            elif k > 3 and _is_channels_last(x) and _convertible(x):
                 # a channels_last trunk: the large dilated kernels only reach tensor-core speed on channel planes, so the
                 # input is re-laid at the block boundary (layout_convert.cu); 3x3 stays on the streaming NHWC kernels
                 layout, in_cl = _abi.NCHW, True

@@ -1,8 +1,6 @@
 """GPU parity tests: the CUDA path (through the C ABI, libkdcc.so) against the CPU oracle and the
 fixtures frozen from the reference modules.  Tolerances are BASELINE.json's: 1e-5 relative in fp32,
 2e-2 in bf16, measured as max|a-b| / max|b| per tensor."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -69,16 +67,9 @@ def test_block_fp32_matches_reference_golden(kdcc, golden_block, tag):
         assert relerr(mine, g[f"{tag}/{name}"]) < TOL[torch.float32], name
 
 
-@pytest.mark.parametrize("mode", ["default", "tma", "tma_plain_load", "tma_plain_store", "direct"])
 @pytest.mark.parametrize("tag", BLOCK_CASES)
-def test_block_bf16_matches_reference_golden(kdcc, golden_block, tag, mode, monkeypatch):
-    # "default": what the dispatcher picks (streaming 3x3 kernels for k=3 d=1 p=1, TMA-staged kernels for k=9);
-    # the tma* modes switch the streaming 3x3 kernels off so that the TMA-staged k=3 configuration stays covered
-    monkeypatch.setenv("KDCC_DW_MODE", {"tma_plain_load": "1", "tma_plain_store": "2"}.get(mode, "0"))
-    monkeypatch.setenv("KDCC_DW_FORCE_DIRECT", "1" if mode == "direct" else "0")
-    monkeypatch.setenv("KDCC_DW_KEEP_NHWC", "1")   # NHWC kernels under test: no re-layout to the NCHW tensor-core path
-    if mode.startswith("tma"):
-        monkeypatch.setenv("KDCC_DW_NHWC3_OFF", "1")
+def test_block_bf16_matches_reference_golden(kdcc, golden_block, tag):
+    # every golden shape has W % 8 != 0, C % 16 != 0 or k <= 3: the channels_last input stays on the NHWC kernels
     g = golden_block
     N, Ci, Co, H, W, k, d, p = [int(v) for v in g[f"{tag}/geom"]]
     y, dx, dwd, dwp = run_block(kdcc, g[f"{tag}/x"], g[f"{tag}/w_dw"], g[f"{tag}/w_pw"], g[f"{tag}/dy"], k, d, p,
@@ -100,20 +91,23 @@ def oracle_block(x, w_dw, w_pw, dy, k, d, p, dtype):
 
 
 SEEDED = [
-    # N, Ci, Co,  H,  W, k, d,  p
-    (2, 64, 128, 40, 40, 9, 5, 20),    # Cityscapes geometry, several 26x26 sub-image tiles
-    (1, 32, 64, 131, 67, 9, 5, 20),    # ragged: residues with unequal sub-image sizes, partial tiles
-    (2, 32, 64, 33, 47, 3, 1, 1),      # 3x3, ragged edges
-    (3, 16, 8, 20, 20, 3, 2, 2),       # dilated 3x3
-    (32, 64, 64, 8, 8, 3, 1, 1),       # CIFAR ResNet44 layer3 block shape
-    (1, 384, 384, 32, 32, 9, 5, 20),   # HRNet-OCR site shape
+    # N, Ci, Co,  H,  W, k, d,  p      (channels_last; bf16 kernel in brackets, fp32 always runs the direct kernels;
+    #                                    k9 widths are not multiples of 8, so the input is not re-laid to planes)
+    (2, 64, 128, 40, 44, 9, 5, 20),    # Cityscapes geometry, several 26x26 sub-image tiles         [TMA k9]
+    (1, 32, 64, 131, 67, 9, 5, 20),    # ragged: residues with unequal sub-image sizes, partial tiles [TMA k9]
+    (2, 32, 64, 33, 47, 3, 1, 1),      # 3x3, ragged edges                                          [streaming 3x3]
+    (3, 16, 8, 20, 20, 3, 2, 2),       # dilated 3x3                                                [TMA k3]
+    (32, 64, 64, 8, 8, 3, 1, 1),       # CIFAR ResNet44 layer3 block shape                          [streaming 3x3]
+    (1, 384, 384, 32, 36, 9, 5, 20),   # HRNet-OCR site channels                                    [TMA k9]
+    (2, 24, 32, 30, 37, 9, 5, 20),     # C % 16 == 8                                                [direct]
+    (2, 24, 48, 20, 20, 3, 1, 1),      # C % 16 == 8                                                [direct]
+    (2, 48, 64, 24, 30, 3, 1, 1),      # six channel vectors: not streamed                          [TMA k3]
 ]
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("geom", SEEDED)
-def test_block_matches_oracle_seeded(kdcc, geom, dtype, monkeypatch):
-    monkeypatch.setenv("KDCC_DW_KEEP_NHWC", "1")   # these cases are about the NHWC kernels: no re-layout to the NCHW path
+def test_block_matches_oracle_seeded(kdcc, geom, dtype):
     N, Ci, Co, H, W, k, d, p = geom
     rs = np.random.RandomState(1234 + Ci + H)
     x = rs.standard_normal((N, Ci, H, W)).astype(np.float32)

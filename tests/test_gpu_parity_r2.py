@@ -346,8 +346,8 @@ def test_wide_planes_run_as_two_column_halves(kdcc, geom):
 def test_depthwise_weight_gradient_column_phase_kernel(kdcc, geom):
     """9 x 9, dilation 5 weight gradient on the column-phase tensor-core kernel (dw_tc_wgrad3.cu: four tap rows per MMA, dy
     transposed by the tensor core) over ragged planes, odd batch sizes and channel counts that split units across CTAs:
-    against torch's fp64 autograd of the reference's depthwise conv (depthwise_separable_conv.py:12) and against the
-    whole-plane kernel it replaces (KDCC_DW_WGRAD_V2=1).  Both operands are exact bf16 and the sums are fp32: 2e-5."""
+    against torch's fp64 autograd of the reference's depthwise conv (depthwise_separable_conv.py:12).  Both operands are
+    exact bf16 and the sums are fp32: 2e-5."""
     n, c, h, w_ = geom
     gen = torch.Generator("cuda").manual_seed(11)
     x = torch.randn(n, c, h, w_, device="cuda", generator=gen).to(torch.bfloat16)
@@ -364,10 +364,4 @@ def test_depthwise_weight_gradient_column_phase_kernel(kdcc, geom):
     torch.nn.functional.conv2d(x.double(), wd, None, 1, 20, 5, c).backward(dy.double())
     ref = wd.grad
     assert ((mine.double() - ref).abs().max() / ref.abs().max()).item() < 2e-5
-    os.environ["KDCC_DW_WGRAD_V2"] = "1"
-    try:
-        old = grad()
-    finally:
-        del os.environ["KDCC_DW_WGRAD_V2"]
-    assert ((mine - old).abs().max() / old.abs().max()).item() < 2e-5
     assert torch.equal(mine, grad())  # deterministic: fixed-order sums, no atomics

@@ -1,9 +1,7 @@
 #!/bin/bash
-# streaming NHWC 3x3: ring lag x CTA shape sweep (variant libraries from tools/build_variant.sh)
+# streaming NHWC 3x3: CTA shape sweep (variant libraries from tools/build_variant.sh)
 P=knowledge-distillation-by-replacing-cheap-conv_b200
 for lib in libkdcc.so libkdcc_w4o3.so libkdcc_w8o1.so; do
   [ -f $P/$lib ] || continue
-  for lag in ${LAGS:-1 2 4 6}; do
-    echo "== $lib lag=$lag: $(KDCC_LIB=$PWD/$P/$lib KDCC_N3_LAG=$lag timeout -s KILL 120 python tools/time_dw_nhwc.py 2>&1 | tail -3 | tr '\n' '|')"
-  done
+  echo "== $lib: $(KDCC_LIB=$PWD/$P/$lib timeout -s KILL 120 python tools/time_dw_nhwc.py 2>&1 | tail -3 | tr '\n' '|')"
 done

@@ -1,8 +1,7 @@
-"""Column-phase depthwise weight gradient (dw_tc_wgrad3.cu) against the whole-plane kernel (KDCC_DW_WGRAD_V2=1) and an fp64
-torch reference, over ragged shapes; then timing of both on the 4096-channel site.  Run on the GPU box."""
+"""Column-phase depthwise weight gradient (dw_tc_wgrad3.cu) against an fp64 torch reference, over ragged shapes; then
+its timing on the 4096-channel site.  Run on the GPU box."""
 import importlib
 import os
-import subprocess
 import sys
 
 import torch
@@ -28,34 +27,18 @@ def ref_grad(x, w, dy):
 
 
 def main():
-    child = os.environ.get("W3_CHILD")
     torch.manual_seed(0)
     dev = "cuda"
     shapes = [(1, 8, 128, 128), (4, 64, 128, 128), (3, 37, 128, 128), (2, 16, 96, 104), (5, 300, 128, 128), (2, 40, 65, 128), (1, 3, 128, 8), (4, 512, 128, 128)]
-    out = {}
     for (n, c, h, w_) in shapes:
         x = torch.randn(n, c, h, w_, device=dev).to(torch.bfloat16)
         dy = torch.randn(n, c, h, w_, device=dev).to(torch.bfloat16)
         w = torch.randn(c, 1, 9, 9, device=dev) * 0.1
-        g = dw_grad(x, w, dy)
-        torch.cuda.synchronize()
-        out[(n, c, h, w_)] = g.cpu()
-        if not child:
-            r = ref_grad(x, w, dy).float().cpu()
-            err = (g.cpu() - r).abs().max().item() / max(r.abs().max().item(), 1e-9)
-            print("shape", (n, c, h, w_), "rel err vs fp64 %.3e" % err, flush=True)
-            assert err < 2e-5, err   # both operands are exact bf16, fp32 accumulation
-    if child:
-        torch.save(out, child)
-        return
-    # same inputs through the previous kernel in a child process
-    path = "/tmp/w3_child.pt"
-    subprocess.run([sys.executable, __file__], env=dict(os.environ, W3_CHILD=path, KDCC_DW_WGRAD_V2="1"), check=True)
-    old = torch.load(path)
-    for k, g in out.items():
-        d = (g - old[k]).abs().max().item() / max(old[k].abs().max().item(), 1e-9)
-        print("shape", k, "rel diff vs wgrad2 %.3e" % d)
-        assert d < 2e-5
+        g = dw_grad(x, w, dy).cpu()
+        r = ref_grad(x, w, dy).float().cpu()
+        err = (g - r).abs().max().item() / max(r.abs().max().item(), 1e-9)
+        print("shape", (n, c, h, w_), "rel err vs fp64 %.3e" % err, flush=True)
+        assert err < 2e-5, err   # both operands are exact bf16, fp32 accumulation
     # timing
     n, c = 4, 4096
     x = torch.randn(n, c, 128, 128, device=dev).to(torch.bfloat16)
