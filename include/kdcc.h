@@ -68,7 +68,10 @@ const char *kdcc_dispatch_name(int op, int N, int H, int W, int C, int Cout, int
 /* ---- depthwise k x k, stride 1, zero padding, dilation `dil` -----------------------------------
  * Replaces self.separable_conv(x)  (models/students/transform_blocks/depthwise_separable_conv.py:7-8,12
  * -> F.conv2d groups=C).  x [N,H,W,C], w fp32 [C,k,k] (the (C,1,k,k) parameter, contiguous),
- * bias fp32 [C] or NULL, y [N,Ho,Wo,C] with Ho = H + 2*pad - dil*(k-1). */
+ * bias fp32 [C] or NULL, y [N,Ho,Wo,C] with Ho = H + 2*pad - dil*(k-1).
+ * layout NCHW (bf16 tensor-core kernels only): odd k <= 9, dil*(k-1) <= 57, W % 8 == 0 and Wo % 8 == 0, and
+ * pad <= dil*(k-1), so that the backward's transposed padding dil*(k-1) - pad is not negative; any other NCHW shape
+ * returns KDCC_ESHAPE here and in kdcc_dw_bwd (kdcc_dispatch_name says "unsupported"), and runs in the NHWC layout. */
 int kdcc_dw_fwd(const void *x, const float *w, const float *bias, void *y, int N, int H, int W, int C,
                 int k, int dil, int pad, int layout, int dtype, kdcc_stream_t stream);
 

@@ -37,10 +37,10 @@ KDCC_API const char *kdcc_dispatch_name(int op, int N, int H, int W, int C, int 
   }
   switch (op) {
     case 0:
-      if (nchw) return bf16 && dw_tc_supported(H, W, Ho, Wo, k, dil) ? "dw_tc_conv" : "unsupported";
+      if (nchw) return bf16 && dw_tc_supported(H, W, Ho, Wo, k, dil, pad) ? "dw_tc_conv" : "unsupported";
       return bf16 && dw_tma_supported(C, k, dil) ? dw_tma_name(k, dil, 0) : "dw_direct";
     case 1:
-      if (nchw) return bf16 && dw_tc_supported(H, W, Ho, Wo, k, dil) ? "dw_tc_wgrad" : "unsupported";
+      if (nchw) return bf16 && dw_tc_supported(H, W, Ho, Wo, k, dil, pad) ? "dw_tc_wgrad" : "unsupported";
       return bf16 && dw_tma_supported(C, k, dil) ? dw_tma_name(k, dil, 1) : "dw_wgrad_direct";
     case 2: case 3: case 4: {
       static const char *names[3] = {"pw_gemm_sm100_fwd", "pw_gemm_sm100_dx", "pw_gemm_sm100_dw"};

@@ -27,7 +27,7 @@ static int check_geometry(int N, int H, int W, int C, int k, int dil, int pad, i
   if (layout == KDCC_LAYOUT_NHWC) {
     if (C % (dtype == KDCC_F32 ? 4 : 8) != 0) return KDCC_ESHAPE;  // 16-byte channel vectors
   } else {
-    if (dtype != KDCC_BF16 || !dw_tc_supported(H, W, *Ho, *Wo, k, dil)) return KDCC_ESHAPE;
+    if (dtype != KDCC_BF16 || !dw_tc_supported(H, W, *Ho, *Wo, k, dil, pad)) return KDCC_ESHAPE;
   }
   return KDCC_OK;
 }
@@ -90,7 +90,6 @@ KDCC_API int kdcc_dw_bwd(const void *x, const float *w, const void *dy, void *dx
   if (layout == KDCC_LAYOUT_NCHW) {
     if (dbias) return KDCC_ESHAPE;  // bias gradients go through kdcc_colsum on the NHWC path
     if (dx) {
-      if (padt < 0) return KDCC_ESHAPE;
       rc = dw_tc_conv(dy, w, nullptr, dx, N, C, Ho, Wo, H, W, k, dil, padt, 1, st);
       if (rc) return rc;
     }

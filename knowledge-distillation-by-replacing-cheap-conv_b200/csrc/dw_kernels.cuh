@@ -34,7 +34,8 @@ int dw_nhwc3_wgrad_ctas(int N, int H, int W, int C);
 int dw_nhwc3_wgrad(const void *x, const void *dy, float *dw, float *part, int N, int H, int W, int C, cudaStream_t st);
 
 // ---- tensor-core (tcgen05) bf16 kernels on NCHW planes: dw_tc.cu, dw_tc_wgrad.cu ---------------------
-bool dw_tc_supported(int Hi, int Wi, int Ho, int Wo, int k, int dil);
+// pad <= dil * (k - 1): the input gradient is the same convolution with the transposed padding dil * (k - 1) - pad
+bool dw_tc_supported(int Hi, int Wi, int Ho, int Wo, int k, int dil, int pad);
 int dw_tc_conv(const void *in, const float *w, const float *bias, void *out, int N, int C, int Hi, int Wi, int Ho,
                int Wo, int k, int dil, int pad, int flip, cudaStream_t st);
 int dw_tc_wgrad(const void *x, const void *dy, float *dw, float *part, int N, int C, int H, int W, int Ho, int Wo,

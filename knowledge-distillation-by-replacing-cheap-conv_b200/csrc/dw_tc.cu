@@ -287,10 +287,11 @@ static int tc_extra(int pad) { return (8 - pad % 8) % 8; }
 // (N + halo + alignment columns) must stay within the instantiated K-slice counts
 static int tc_nt(int reach) { return reach + 32 <= 80 ? 32 : 16; }
 
-bool dw_tc_supported(int Hi, int Wi, int Ho, int Wo, int k, int dil) {
+bool dw_tc_supported(int Hi, int Wi, int Ho, int Wo, int k, int dil, int pad) {
   (void)Hi; (void)Ho;
   const int halo = dil * (k - 1);
   if (k > 9 || k % 2 == 0) return false;      // wgrad keeps k*k register partials: instantiated for k = 1,3,5,7,9
+  if (pad > halo) return false;               // the input gradient runs this kernel with pad' = halo - pad >= 0
   if (halo + 7 + 16 > 80) return false;       // Toeplitz K extent (incl. alignment columns) <= 5 slices of 16
   if (Wi % 8 != 0 || Wo % 8 != 0) return false;  // 16-byte rows for TMA strides and epilogue stores
   return true;

@@ -130,7 +130,6 @@ KDCC_API int kdcc_pw_bwd_dw(const void *dy, const void *x, float *dw, void *work
   rc = dtype == KDCC_BF16 ? pw_simt_gemm<__nv_bfloat16>(dy, x, g, st) : pw_simt_gemm<float>(dy, x, g, st);
   if (rc || g.splits == 1) return rc;
   const long count = (long)Nc * K;
-  if (count % 4 != 0) return KDCC_ESHAPE;
-  reduce_splits_kernel<<<(unsigned)ceil_div<long>(count / 4, 256), 256, 0, st>>>(part, dw, g.splits, count);
+  reduce_splits_kernel<<<(unsigned)ceil_div<long>(count, 4 * 256), 256, 0, st>>>(part, dw, g.splits, count);
   return launch_status();
 }

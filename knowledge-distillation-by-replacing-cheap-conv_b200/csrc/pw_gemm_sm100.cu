@@ -352,11 +352,19 @@ pw_gemm_sm100_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
   }
 }
 
-// out[i] = sum_s part[s][i]   (fixed order)
+// out[i] = sum_s part[s][i]   (fixed order); four elements per thread, as float4 when count % 4 == 0 keeps them aligned
 __global__ void reduce_splits_kernel(const float *__restrict__ part, float *__restrict__ out, int splits, long count) {
   pdl_prologue_done();
   const long i4 = ((long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (i4 >= count) return;
+  if (count % 4 != 0) {  // the CUDA-core fp32 / odd-channel weight gradient: Nc * K of any value
+    for (long i = i4; i < i4 + 4 && i < count; ++i) {
+      float acc = 0.f;
+      for (int s = 0; s < splits; ++s) acc += part[(long)s * count + i];
+      out[i] = acc;
+    }
+    return;
+  }
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int s = 0; s < splits; ++s) {
     const float4 v = *reinterpret_cast<const float4 *>(part + (long)s * count + i4);

@@ -1,6 +1,7 @@
 """Which kernel runs for which arguments: forward + backward under torch.profiler, launched kernel names against the
 table below.  The library picks its kernels from the call's arguments alone, so the parity tests prove a kernel by
-the shapes that reach it; this table keeps those shapes reaching it.  It is the only place a test names a kernel."""
+the shapes that reach it; this table keeps those shapes reaching it.  It and test_conv_edges.py, whose parity rows pin
+the kernels of every shape they run, are the only places a test names a kernel."""
 import re
 
 import pytest
